@@ -356,6 +356,25 @@ def emit(line: dict):
     out.flush()
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def snapshot(**arrays) -> dict:
+    """float64 C-ordered copies of what a step returned: the passes after the timed one overwrite the same host buffers."""
+    return {k: np.array(v, dtype=np.float64, order="C", ndmin=1) for k, v in arrays.items()}
+
+
+def dump_outputs(path: str, arrays: dict):
+    """--dump-outputs: the last timed step's results as DIR/<name>.npy, so that two builds run on the same seeded inputs can be
+    compared output for output."""
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def setup_dist(args):
     # stdout carries exactly one JSON line.  NCCL logs to the process's stdout (its version banner at any NCCL_DEBUG level), so file
     # descriptor 1 is pointed at stderr for the lifetime of the process and the JSON line goes to a duplicate of the original stdout.
@@ -510,6 +529,7 @@ def run_svgp(args, w):
     clk = clocks.stop() if clocks else {}
     launches = ctx.launch_count() - l0
     value = N_total * args.steps / (ms * 1e-3)
+    last = snapshot(elbo=out.value, **{"grad_" + k: v for k, v in gb.items()})
 
     # ---- profiled pass: per-kernel-class CUDA-event times of the same steps (not part of `value`) -------
     psteps = 1 if w.get("long_step") else max(1, min(args.steps, 3))
@@ -659,6 +679,8 @@ def run_svgp(args, w):
                                    "elbo_rel": abs(out.value - ref) / abs(ref), "grad_rel_to_max": errs, "tol": 1e-4 if f32 else 1e-10,
                                    "ok": bool(abs(out.value - ref) / abs(ref) < (1e-4 if f32 else 1e-10) and max(errs.values()) < (1e-4 if f32 else 1e-10))}
         emit(line)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, last)
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
@@ -696,6 +718,7 @@ def run_laplace(args, w):
     clk = clocks.stop() if clocks else {}
     launches = ctx.launch_count() - l0
     r = res["r"]
+    last = snapshot(f_opt=r.f, lml=r.lml, newton_steps=r.steps)
     iters = r.steps + (0 if r.converged else 1)  # a converged loop reuses its last cache for the lml (DESIGN.md section 2)
     it_per_s = world * iters * args.steps / (ms * 1e-3)
     ms_iter = ms / args.steps / iters
@@ -747,6 +770,8 @@ def run_laplace(args, w):
             line["cpu_baseline"] = {"value": gflops * 1e9 / flop_it, "unit": LAPLACE_UNIT, "cores": host_threads(), "kind": "port", "gflops": gflops,
                                     "sample": f"the same recipe at n={n_cpu} ({steps + 1} Newton iterations, median of 3: {t:.2f} s), extrapolated to N={n} by n^3/3 + 6 n^2"}
         emit(line)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, last)
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
@@ -842,6 +867,8 @@ def run_c1(args, w):
         ms = timed(epoch, args.steps)
         clk = clocks.stop() if clocks else {}
         launches = ctx.launch_count() - l0
+        if M == w["M"]:  # the evaluation `value` is quoted on: the last minibatch of the last timed epoch
+            last = snapshot(elbo=out.value, grad_flat=g)
         t0 = time.perf_counter()
         for _ in range(args.steps):
             epoch()
@@ -881,6 +908,8 @@ def run_c1(args, w):
                                     "sample": f"300 minibatch evaluations per M, NumPy/SciPy OpenBLAS threads={host_threads()}",
                                     "us_per_evaluation": {f"M{m}": 1e6 / v for m, v in cpu.items()}}
         emit(line)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, last)
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
@@ -899,7 +928,13 @@ def main():
     ap.add_argument("--no-check", action="store_true", help="skip the N > 1 sharded-vs-single-rank correctness evaluation")
     ap.add_argument("--dtype", default="f64", choices=["f64", "f32", "f32_tc_solve", "f64emu"], help="f64emu: Float64 tolerance with S6 as an FP64-accurate INT8-slice product on tcgen05 (AGP_COMPUTE_F64_EMU; its own line, never the headline); f32: the Float32 fast mode (3xTF32 on tcgen05 for the GEMM-shaped sweep stages); "
                                                                              "reported as its own line, never as the Float64 headline")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned (ELBO and gradients; Laplace: f_opt, lml) as DIR/<name>.npy, float64")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs records the b200 arm's outputs")
     w = dict(WORKLOADS[args.workload])
     if args.n:
         w["N"] = args.n
