@@ -155,23 +155,13 @@ struct Prof {
 
 static void lap_release(agp_ctx* c);
 static void chol_partition_release(agp_ctx* c);
-// AGP_F64_EMU_S2=0 keeps S2 of AGP_COMPUTE_F64_EMU on the DMMA kernel (A/B knob)
-static bool f64_emu_s2() {
-  static const bool off = getenv("AGP_F64_EMU_S2") && atoi(getenv("AGP_F64_EMU_S2")) == 0;
-  return !off;
-}
-// AGP_F64_S6=i8 forces AGP_COMPUTE_F64_EMU (S6 as an FP64-accurate 7-slice INT8 product) on every Float64 evaluation of the process: A/B knob
-static bool f64_s6_i8() {
-  static const bool on = getenv("AGP_F64_S6") && strcmp(getenv("AGP_F64_S6"), "i8") == 0;
-  return on;
-}
 struct agp_ctx {
   Prof prof;
   void* lap = nullptr;  // LapWork (laplace_host.inc)
   int device = 0;
   cudaStream_t stream = nullptr;
   cudaStream_t stream2 = nullptr;                // trailing updates of the blocked Cholesky (look-ahead), see blocked_cholesky
-  cudaEvent_t ev_panel = nullptr, ev_trail = nullptr;
+  cudaEvent_t ev_trail = nullptr;
   cudaStream_t stream3 = nullptr;                // tile-level look-ahead of the blocked Cholesky: full-height panels / in-super-panel updates
   // SM partition for large factorisations (green contexts, see chol_partition): the critical chain on its own 8 SMs
   int part_state = 0;                            // 0 = not tried, 1 = in use, -1 = unavailable
@@ -179,7 +169,7 @@ struct agp_ctx {
   cudaStream_t pstream_chain = nullptr, pstream_side = nullptr, pstream_trail = nullptr;
   cudaEvent_t ev_enter = nullptr, ev_leave = nullptr;
   int part_sms_chain = 0, part_sms_bulk = 0;
-  cudaEvent_t ev_diag = nullptr, ev_prow = nullptr, ev_side = nullptr, ev_prio[4] = {nullptr, nullptr, nullptr, nullptr};
+  cudaEvent_t ev_diag = nullptr, ev_prow = nullptr, ev_side = nullptr, ev_prio = nullptr;
   cudaStream_t stream_copy = nullptr;            // upload of the q.Sigma factor (M^2 doubles) behind the Kuu factorisation, see prepare_step
   cudaEvent_t ev_copy = nullptr;
   int sms = 148;
@@ -194,7 +184,7 @@ struct agp_ctx {
   // accumulators
   DevBuf gpart, Gpart, kpart, red, small, ghbuf;
   DevBuf qBt7, sBt7, sPm;  // AGP_COMPUTE_F64_EMU, S2: slices / scales of Bt^T (once per sweep), per-point scales of the point-major slices of A
-  DevBuf q6A, q6As, s6;  // Float64 mode, S6 on the INT8 tensor path (experiment knob AGP_F64_S6=i8): slice planes of A and As, [scales A | scales As | row maxima x 2]
+  DevBuf q6A, q6As, s6;  // AGP_COMPUTE_F64_EMU, S6 on the INT8 tensor path: slice planes of A and As, [scales A | scales As | row maxima x 2]
   // Float32 mode: hi | lo FP32 planes (each DevBuf holds both: 2 x count floats = count doubles)
   DevBuf fA, fC, fAb, fAs, fBtc, fBtr, fLi;
   DevBuf qAb, sAb, qLi, sLi;
@@ -258,12 +248,11 @@ extern "C" int32_t agp_ctx_create(int32_t device, agp_ctx** out) {
   CU(cudaStreamCreateWithPriority(&c->stream, cudaStreamNonBlocking, prio_hi));
   CU(cudaStreamCreateWithPriority(&c->stream2, cudaStreamNonBlocking, prio_lo));
   CU(cudaStreamCreateWithPriority(&c->stream3, cudaStreamNonBlocking, prio_hi < prio_lo - 1 ? prio_hi + 1 : prio_hi));
-  CU(cudaEventCreateWithFlags(&c->ev_panel, cudaEventDisableTiming));
   CU(cudaEventCreateWithFlags(&c->ev_trail, cudaEventDisableTiming));
   CU(cudaEventCreateWithFlags(&c->ev_diag, cudaEventDisableTiming));
   CU(cudaEventCreateWithFlags(&c->ev_prow, cudaEventDisableTiming));
   CU(cudaEventCreateWithFlags(&c->ev_side, cudaEventDisableTiming));
-  for (int i = 0; i < 4; i++) CU(cudaEventCreateWithFlags(&c->ev_prio[i], cudaEventDisableTiming));
+  CU(cudaEventCreateWithFlags(&c->ev_prio, cudaEventDisableTiming));
   CU(cudaStreamCreateWithFlags(&c->stream_copy, cudaStreamNonBlocking));
   CU(cudaEventCreateWithFlags(&c->ev_copy, cudaEventDisableTiming));
   CU(cudaMalloc(&c->d_flags, 4 * sizeof(int)));
@@ -285,10 +274,9 @@ extern "C" int32_t agp_ctx_destroy(agp_ctx* c) {
   lap_release(c);
   if (c->d_flags) cudaFree(c->d_flags);
   for (cudaEvent_t e : c->prof.pool) cudaEventDestroy(e);
-  if (c->ev_panel) cudaEventDestroy(c->ev_panel);
   if (c->ev_trail) cudaEventDestroy(c->ev_trail);
   if (c->stream2) cudaStreamDestroy(c->stream2);
-  for (cudaEvent_t e : {c->ev_diag, c->ev_prow, c->ev_side, c->ev_prio[0], c->ev_prio[1], c->ev_prio[2], c->ev_prio[3]})
+  for (cudaEvent_t e : {c->ev_diag, c->ev_prow, c->ev_side, c->ev_prio})
     if (e) cudaEventDestroy(e);
   if (c->stream3) cudaStreamDestroy(c->stream3);
   chol_partition_release(c);
@@ -611,8 +599,7 @@ static int32_t run_gemm(agp_ctx* c, int tiles_m, int tiles_n, const double* A, i
   OK((ensure_smem<gemm_kernel<LA, LB, Epi, S>>(c, smem_bytes)));
   dim3 grid(tiles_m, tiles_n);
   if ((kmode == KR_LOWER || kmode == KR_UPPER) && tmode == TS_ALL && tiles_m > 1) {
-    static const int env_g = getenv("AGP_SWIZZLE") ? atoi(getenv("AGP_SWIZZLE")) : 0;  // tuning knob
-    g.swizzle = env_g > 0 ? env_g : std::max(1, c->sms);  // half a wave of column tiles per super-group
+    g.swizzle = std::max(1, c->sms);  // half a wave of column tiles per super-group
     g.tiles_m = tiles_m;
     g.tiles_n = tiles_n;
     grid = dim3(tiles_m * tiles_n, 1);
@@ -659,112 +646,13 @@ static int32_t transpose(agp_ctx* c, const double* in, double* out, int n, int64
   return AGP_OK;
 }
 
-// Two-level blocked right-looking Cholesky of the n x n (n = nb*128) matrix Kw (column-major, lower triangle read,
-// destroyed) into L; also produces the inverse diagonal blocks in the diagonal blocks of Lt (inv) and Ut (inv^T).
-// Inner level: 128-blocks (diagonal kernel + panel GEMM + an update confined to the current 512-wide super-panel);
-// outer level: one trailing update per super-panel with K = 512, which quadruples the flop per byte of the
-// dominant GEMM compared with a rank-128 update.
-// Look-ahead: the factorisation of a super-panel is a chain of latency-bound launches (one CTA on the diagonal block,
-// then a few dozen GEMM tiles) that leaves the machine idle, while the trailing update is the only part with enough tiles
-// to fill it.  So the trailing update is split: the block columns of the NEXT super-panel are updated on the main stream
-// (the chain continues with them at once), the remaining columns on a second stream, concurrently with the next
-// super-panel's chain.  The arithmetic of every tile is unchanged (same k order), so the factor is bit-identical to the
-// single-stream schedule.
-struct StreamSwap {  // launch helpers use c->stream: point it at the second stream for a scope
+// launch helpers use c->stream: point it at another stream for a scope
+struct StreamSwap {
   agp_ctx* c;
   cudaStream_t saved;
   StreamSwap(agp_ctx* c_, cudaStream_t s) : c(c_), saved(c_->stream) { c->stream = s; }
   ~StreamSwap() { c->stream = saved; }
 };
-static int32_t blocked_cholesky_v2(agp_ctx* c, double* Kw, double* L, double* Lt, double* Ut, int nb, int64_t ld, int* info, int nvalid);
-static int32_t blocked_cholesky(agp_ctx* c, double* Kw, double* L, double* Lt, double* Ut, int nb, int64_t ld, int* info, int nvalid) {
-  // AGP_CHOL_SCHED=1 selects the super-panel-level look-ahead of round 1 (kept for A/B measurements); the default is the tile-level one
-  static const int sched = getenv("AGP_CHOL_SCHED") ? atoi(getenv("AGP_CHOL_SCHED")) : 2;
-  if (sched == 2 && nb > 1) return blocked_cholesky_v2(c, Kw, L, Lt, Ut, nb, ld, info, nvalid);
-  OK((ensure_smem<potrf_trinv128_kernel>(c, PT_SMEM_BYTES)));
-  constexpr int OB = 4;  // inner blocks per super-panel
-  static const bool lookahead = !(getenv("AGP_CHOL_LOOKAHEAD") && atoi(getenv("AGP_CHOL_LOOKAHEAD")) == 0);  // tuning knob
-  bool trail_pending = false;  // a trailing update is in flight on stream2
-  // development aid (AGP_CHOL_TRACE=1): device timestamps of the phases of one large factorisation, printed to stderr
-  static int trace_left = (getenv("AGP_CHOL_TRACE") && nb >= 32) ? 1 : 0;
-  const bool trace = trace_left > 0 && nb >= 32;
-  struct Mark { const char* what; int s; cudaEvent_t e; };
-  std::vector<Mark> marks;
-  auto mark = [&](const char* what, int s, cudaStream_t st) {
-    if (!trace) return;
-    cudaEvent_t e;
-    cudaEventCreate(&e);
-    cudaEventRecord(e, st);
-    marks.push_back({what, s, e});
-  };
-  mark("start", 0, c->stream);
-  for (int J0 = 0; J0 < nb; J0 += OB) {
-    const int J1 = std::min(nb, J0 + OB);  // super-panel = block columns [J0, J1)
-    for (int J = J0; J < J1; J++) {
-      const int64_t djj = (int64_t)J * BM * ld + (int64_t)J * BM;
-      potrf_trinv128_kernel<<<1, 256, PT_SMEM_BYTES, c->stream>>>(Kw + djj, L + djj, Lt + djj, Ut + djj, ld, J * BM, info, std::max(0, std::min(BM, nvalid - J * BM)));
-      LAUNCHED(c);
-      KCHECK();
-      const int rem = nb - 1 - J;
-      if (rem == 0) break;
-      const int64_t pnl = (int64_t)J * BM * ld + (int64_t)(J + 1) * BM;  // block column J, rows below the diagonal block
-      // panel: L[>J, J] = Kw[>J, J] * inv(L_JJ)^T ;  B(k, n) = inv[n][k] = Lt[djj + n + k*ld]
-      OK((run_gemm<A_KM, B_KN>(c, rem, 2, Kw + pnl, ld, Lt + djj, ld, BM, KR_FULL, TS_ALL, epi_store(L + pnl, ld, false))));
-      // update of the remaining block columns (J, J1) of this super-panel (lower tiles): Kw[>J, J+1..J1) -= P P^T
-      const int wcols = J1 - 1 - J;
-      if (wcols > 0) {
-        const int64_t trl = (int64_t)(J + 1) * BM * ld + (int64_t)(J + 1) * BM;
-        OK((run_gemm<A_KM, B_KN>(c, rem, 2 * wcols, L + pnl, ld, L + pnl, ld, BM, KR_FULL, TS_NBLK_LE, epi_store(Kw + trl, ld, false, -1.0, 1.0))));
-      }
-    }
-    const int rem = nb - J1;
-    if (rem <= 0) break;
-    // trailing update with the whole super-panel: Kw[>=J1, >=J1] -= L[>=J1, J0..J1) L[>=J1, J0..J1)^T
-    const int K = (J1 - J0) * BM;
-    const int64_t pnl = (int64_t)J0 * BM * ld + (int64_t)J1 * BM;
-    const int64_t trl = (int64_t)J1 * BM * ld + (int64_t)J1 * BM;
-    const int J2 = std::min(nb, J1 + OB), rem2 = nb - J2;  // [J1, J2) = the next super-panel
-    if (!lookahead || rem2 <= 0) {
-      if (trail_pending) CU(cudaStreamWaitEvent(c->stream, c->ev_trail, 0));
-      trail_pending = false;
-      OK((run_gemm<A_KM, B_KN>(c, rem, 2 * rem, L + pnl, ld, L + pnl, ld, K, KR_FULL, TS_NBLK_LE, epi_store(Kw + trl, ld, false, -1.0, 1.0))));
-      continue;
-    }
-    CU(cudaEventRecord(c->ev_panel, c->stream));  // block columns [J0, J1) of L are complete
-    mark("factor_done", J0 / OB, c->stream);
-    // main stream: columns [J1, J2) only (they were last written by the previous trailing update on stream2)
-    if (trail_pending) CU(cudaStreamWaitEvent(c->stream, c->ev_trail, 0));
-    mark("prio_start", J0 / OB, c->stream);
-    OK((run_gemm<A_KM, B_KN>(c, rem, 2 * (J2 - J1), L + pnl, ld, L + pnl, ld, K, KR_FULL, TS_NBLK_LE, epi_store(Kw + trl, ld, false, -1.0, 1.0))));
-    mark("prio_done", J0 / OB, c->stream);
-    {  // second stream: columns >= J2 (stream order serialises successive trailing updates of the same tiles)
-      StreamSwap sw(c, c->stream2);
-      CU(cudaStreamWaitEvent(c->stream, c->ev_panel, 0));
-      mark("trail_start", J0 / OB, c->stream);
-      const int64_t pnl2 = (int64_t)J0 * BM * ld + (int64_t)J2 * BM;
-      const int64_t trl2 = (int64_t)J2 * BM * ld + (int64_t)J2 * BM;
-      // 2-stage instantiation (51 KB per CTA): a finished CTA leaves room for the diagonal kernel (166 KB) on its SM
-      OK((run_gemm<A_KM, B_KN, 2>(c, rem2, 2 * rem2, L + pnl2, ld, L + pnl2, ld, K, KR_FULL, TS_NBLK_LE, epi_store(Kw + trl2, ld, false, -1.0, 1.0))));
-      CU(cudaEventRecord(c->ev_trail, c->stream));
-      mark("trail_done", J0 / OB, c->stream);
-      trail_pending = true;
-    }
-  }
-  if (trail_pending) CU(cudaStreamWaitEvent(c->stream, c->ev_trail, 0));
-  if (trace) {
-    mark("end", 0, c->stream);
-    trace_left = 0;
-    cudaStreamSynchronize(c->stream);
-    cudaStreamSynchronize(c->stream2);
-    for (const Mark& m : marks) {
-      float ms = 0.f;
-      cudaEventElapsedTime(&ms, marks[0].e, m.e);
-      fprintf(stderr, "[chol trace] %-12s s=%2d t=%9.1f us\n", m.what, m.s, 1e3 * ms);
-    }
-    for (const Mark& m : marks) cudaEventDestroy(m.e);
-  }
-  return AGP_OK;
-}
 
 // ---- SM partition for the blocked Cholesky (CUDA green contexts) ---------------------------------------------------------
 // The chain of a large factorisation (diagonal-block kernel -> block row of the panel -> tile update -> next diagonal block) is a
@@ -802,7 +690,7 @@ static GreenApi& green_api() {
 static bool chol_partition(agp_ctx* c) {
   if (c->part_state != 0) return c->part_state > 0;
   c->part_state = -1;
-  if (getenv("AGP_CHOL_PARTITION") && atoi(getenv("AGP_CHOL_PARTITION")) == 0) return false;  // A/B knob
+  if (getenv("AGP_CHOL_PARTITION") && atoi(getenv("AGP_CHOL_PARTITION")) == 0) return false;  // for profilers that cannot follow green-context streams
   GreenApi& g = green_api();
   if (!g.ok) return false;
   CUdevice dev;
@@ -864,19 +752,30 @@ static void chol_partition_release(agp_ctx* c) {
   c->part_state = -1;
 }
 
-// Tile-level look-ahead (round 2).  The schedule above keeps the whole chain diag(J) -> panel(J) -> update(J) on one stream, so that the
-// 128 x 128 diagonal kernel of block J+1 (one CTA, ~80 us) waits for two full-height GEMM launches it does not depend on, and the next
-// super-panel waits for all four of its block columns to receive the K = 512 update.  diag(J+1) needs only block row J+1: the panel tile
-// L[J+1,J] = Kw[J+1,J] inv(L_JJ)^T and the update of Kw[J+1,J+1].  So:
-//   main stream (highest priority): diag(J), row J+1 of the panel (2 CTAs), update of the (J+1,J+1) tile (2 CTAs; K = 512 from the whole
-//                                   previous super-panel when J+1 opens a new one), diag(J+1), ...
+// Two-level blocked right-looking Cholesky of the n x n (n = nb*128) matrix Kw (column-major, lower triangle read,
+// destroyed) into L; also produces the inverse diagonal blocks in the diagonal blocks of Lt (inv) and Ut (inv^T).
+// Inner level: 128-blocks (diagonal kernel + panel GEMM + an update confined to the current 512-wide super-panel);
+// outer level: one trailing update per super-panel with K = 512, which quadruples the flop per byte of the
+// dominant GEMM compared with a rank-128 update.
+// Tile-level look-ahead.  The factorisation is a chain of latency-bound launches (one CTA on the diagonal block, ~80 us, then a few GEMM
+// tiles), while the trailing updates are the only part with enough tiles to fill the machine.  diag(J+1) needs only block row J+1: the
+// panel tile L[J+1,J] = Kw[J+1,J] inv(L_JJ)^T and the update of Kw[J+1,J+1], not the full-height GEMMs of block column J; nor does the
+// next super-panel wait for all four of its block columns to receive the K = 512 update.  So:
+//   main stream (highest priority): diag(J), row J+1 of the panel, update of the (J+1,J+1) tile (K = 512 from the whole previous
+//                                   super-panel when J+1 opens a new one), diag(J+1), ...  -- the row products as chain_gemm32_kernel tiles
 //   side stream (middle priority):  rows >= J+2 of panel(J) and of the in-super-panel update, then -- at the end of a super-panel -- the
-//                                   K = 512 update of the next super-panel's block columns, one launch per column in the order in
-//                                   which the chain consumes them
-//   trail stream (lowest priority): the K = 512 update of all later columns (2-stage tiles, as before)
-// Every output tile is produced by the same k loop as in the one-stream schedule, so the factor is bit-identical to it.
-static int32_t blocked_cholesky_v2(agp_ctx* c, double* Kw, double* L, double* Lt, double* Ut, int nb, int64_t ld, int* info, int nvalid) {
+//                                   K = 512 update of the next super-panel's block columns
+//   trail stream (lowest priority): the K = 512 update of all later columns
+// The side-stream and trailing GEMMs use 4-stage tiles: 29 against 24 TFLOP/s for 2-stage ones.
+// Every output tile is produced by the same k loop as in a one-stream schedule, so the factor is bit-identical to it.
+static int32_t blocked_cholesky(agp_ctx* c, double* Kw, double* L, double* Lt, double* Ut, int nb, int64_t ld, int* info, int nvalid) {
   OK((ensure_smem<potrf_trinv128_kernel>(c, PT_SMEM_BYTES)));
+  if (nb == 1) {
+    potrf_trinv128_kernel<<<1, 256, PT_SMEM_BYTES, c->stream>>>(Kw, L, Lt, Ut, ld, 0, info, std::min(BM, nvalid));
+    LAUNCHED(c);
+    KCHECK();
+    return AGP_OK;
+  }
   constexpr int OB = 4;  // inner blocks per super-panel
   cudaStream_t sm = c->stream, ss = c->stream3, st = c->stream2;
   cudaStream_t caller = c->stream;
@@ -893,13 +792,6 @@ static int32_t blocked_cholesky_v2(agp_ctx* c, double* Kw, double* L, double* Lt
   StreamSwap chain_scope(c, sm);  // launch helpers use c->stream
   auto at = [&](int r, int col) { return (int64_t)col * BM * ld + (int64_t)r * BM; };  // offset of block (r, col)
   bool trail_pending = false, prio_pending = false;
-  int prio_cols = 0;
-  static const bool small_tiles = !(getenv("AGP_CHOL_SMALLTILES") && atoi(getenv("AGP_CHOL_SMALLTILES")) == 0);  // A/B knob: chain_gemm32_kernel
-  static const int t4 = getenv("AGP_CHOL_T4") ? atoi(getenv("AGP_CHOL_T4")) : 0;  // A/B knob: 4-stage trailing tiles while rem2 >= t4 (2-stage below)
-  // A/B knobs kept from the measurements: 2-stage tiles (51 KB) for the side-stream / trailing GEMMs.  They were introduced so that one
-  // finished CTA leaves room for the 166 KB diagonal kernel; the traces showed that placement was never the problem (the diagonal kernel
-  // was slow because it SHARED its SM with DMMA tiles), and 4-stage tiles are 29 against 24 TFLOP/s, so both default to 4 stages.
-  static const bool side2 = getenv("AGP_CHOL_SIDE2") && atoi(getenv("AGP_CHOL_SIDE2")) != 0;
   // development aid (AGP_CHOL_TRACE=1): device timestamps around every diagonal-block kernel of one large factorisation
   static int trace_left = getenv("AGP_CHOL_TRACE") ? 3 : 0;  // the third large factorisation of the process (warm) is traced
   if (trace_left > 0 && nb >= 32) trace_left--;
@@ -926,38 +818,27 @@ static int32_t blocked_cholesky_v2(agp_ctx* c, double* Kw, double* L, double* Lt
       const int below = nb - 1 - J;  // block rows J+1 .. nb-1
       // ---- main stream: block row J+1 ----
       if (J > J0) CU(cudaStreamWaitEvent(sm, c->ev_side, 0));  // side(J-1): Kw[J+1, J] and Kw[J+1, J+1] carry update(J-1)
-      else if (prio_pending) CU(cudaStreamWaitEvent(sm, c->ev_prio[0], 0));  // K = 512 update of this super-panel's block columns
-      if (small_tiles) {
-        chain_gemm32_kernel<<<dim3(4, 4), 128, 0, sm>>>(Kw + at(J + 1, J), ld, Lt + at(J, J), ld, BM, 1, 0, L + at(J + 1, J), ld, 1.0, 0.0);
-        LAUNCHED(c);
-        KCHECK();
-      } else {
-        OK((run_gemm<A_KM, B_KN>(c, 1, 2, Kw + at(J + 1, J), ld, Lt + at(J, J), ld, BM, KR_FULL, TS_ALL, epi_store(L + at(J + 1, J), ld, false))));
-      }
+      else if (prio_pending) CU(cudaStreamWaitEvent(sm, c->ev_prio, 0));  // K = 512 update of this super-panel's block columns
+      chain_gemm32_kernel<<<dim3(4, 4), 128, 0, sm>>>(Kw + at(J + 1, J), ld, Lt + at(J, J), ld, BM, 1, 0, L + at(J + 1, J), ld, 1.0, 0.0);
+      LAUNCHED(c);
+      KCHECK();
       CU(cudaEventRecord(c->ev_prow, sm));
       if (J + 1 < J1) {
-        if (small_tiles) {
-          chain_gemm32_kernel<<<dim3(4, 4), 128, 0, sm>>>(L + at(J + 1, J), ld, L + at(J + 1, J), ld, BM, 0, 1, Kw + at(J + 1, J + 1), ld, -1.0, 1.0);
-          LAUNCHED(c);
-          KCHECK();
-        } else {
-          OK((run_gemm<A_KM, B_KN>(c, 1, 2, L + at(J + 1, J), ld, L + at(J + 1, J), ld, BM, KR_FULL, TS_ALL, epi_store(Kw + at(J + 1, J + 1), ld, false, -1.0, 1.0))));
-        }
+        chain_gemm32_kernel<<<dim3(4, 4), 128, 0, sm>>>(L + at(J + 1, J), ld, L + at(J + 1, J), ld, BM, 0, 1, Kw + at(J + 1, J + 1), ld, -1.0, 1.0);
+        LAUNCHED(c);
+        KCHECK();
       }
       // ---- side stream: rows >= J+2 of panel(J) and of the update of the remaining block columns (J, J1) ----
       {
         StreamSwap sw(c, ss);
         CU(cudaStreamWaitEvent(ss, c->ev_diag, 0));
         if (below > 1) {
-          if (side2) OK((run_gemm<A_KM, B_KN, 2>(c, below - 1, 2, Kw + at(J + 2, J), ld, Lt + at(J, J), ld, BM, KR_FULL, TS_ALL, epi_store(L + at(J + 2, J), ld, false))));
-          else OK((run_gemm<A_KM, B_KN>(c, below - 1, 2, Kw + at(J + 2, J), ld, Lt + at(J, J), ld, BM, KR_FULL, TS_ALL, epi_store(L + at(J + 2, J), ld, false))));
+          OK((run_gemm<A_KM, B_KN>(c, below - 1, 2, Kw + at(J + 2, J), ld, Lt + at(J, J), ld, BM, KR_FULL, TS_ALL, epi_store(L + at(J + 2, J), ld, false))));
           const int wcols = J1 - 1 - J;
           if (wcols > 0) {
             CU(cudaStreamWaitEvent(ss, c->ev_prow, 0));  // L[J+1, J] is an operand of column J+1's tiles
-            if (side2) OK((run_gemm<A_KM, B_KN, 2>(c, below - 1, 2 * wcols, L + at(J + 2, J), ld, L + at(J + 1, J), ld, BM, KR_FULL, TS_NBLK_LE1,
-                                                epi_store(Kw + at(J + 2, J + 1), ld, false, -1.0, 1.0))));
-            else OK((run_gemm<A_KM, B_KN>(c, below - 1, 2 * wcols, L + at(J + 2, J), ld, L + at(J + 1, J), ld, BM, KR_FULL, TS_NBLK_LE1,
-                                          epi_store(Kw + at(J + 2, J + 1), ld, false, -1.0, 1.0))));
+            OK((run_gemm<A_KM, B_KN>(c, below - 1, 2 * wcols, L + at(J + 2, J), ld, L + at(J + 1, J), ld, BM, KR_FULL, TS_NBLK_LE1,
+                                     epi_store(Kw + at(J + 2, J + 1), ld, false, -1.0, 1.0))));
           }
         }
         CU(cudaEventRecord(c->ev_side, ss));
@@ -970,37 +851,29 @@ static int32_t blocked_cholesky_v2(agp_ctx* c, double* Kw, double* L, double* Lt
     // ---- main stream: the diagonal block that opens the next super-panel.  L[J1, J0..J1-2] came from the side stream (the main stream
     // has waited for side(J1-2) above), L[J1, J1-1] from the main stream itself.
     if (trail_pending) CU(cudaStreamWaitEvent(sm, c->ev_trail, 0));
-    if (small_tiles) {
-      chain_gemm32_kernel<<<dim3(4, 4), 128, 0, sm>>>(L + at(J1, J0), ld, L + at(J1, J0), ld, K, 0, 1, Kw + at(J1, J1), ld, -1.0, 1.0);
-      LAUNCHED(c);
-      KCHECK();
-    } else {
-      OK((run_gemm<A_KM, B_KN>(c, 1, 2, L + at(J1, J0), ld, L + at(J1, J0), ld, K, KR_FULL, TS_ALL, epi_store(Kw + at(J1, J1), ld, false, -1.0, 1.0))));
-    }
+    chain_gemm32_kernel<<<dim3(4, 4), 128, 0, sm>>>(L + at(J1, J0), ld, L + at(J1, J0), ld, K, 0, 1, Kw + at(J1, J1), ld, -1.0, 1.0);
+    LAUNCHED(c);
+    KCHECK();
     // ---- trail stream: columns >= J2 (needs every row >= J2 of block columns [J0, J1): the side stream up to side(J1-1)) ----
     const int rem2 = nb - J2;
-    // ---- side stream: block columns [J1, J2), one launch each ----
+    // ---- side stream: block columns [J1, J2) ----
     {
       StreamSwap sw(c, ss);
       CU(cudaStreamWaitEvent(ss, c->ev_prow, 0));  // L[J1, J1-1]
       if (trail_pending) CU(cudaStreamWaitEvent(ss, c->ev_trail, 0));  // these columns were last written by the previous trailing update
-      prio_cols = J2 - J1;
+      const int prio_cols = J2 - J1;
       // rows >= J1+1 of the block columns [J1, J2) in one launch (a single wave of tiles once few rows are left: the per-column launches
       // tried first kept the side stream busy for four tile durations and the chain waited for side(J1) behind them)
       if (rem > 1) {
-        if (side2) OK((run_gemm<A_KM, B_KN, 2>(c, rem - 1, 2 * prio_cols, L + at(J1 + 1, J0), ld, L + at(J1, J0), ld, K, KR_FULL, TS_NBLK_LE1, epi_store(Kw + at(J1 + 1, J1), ld, false, -1.0, 1.0))));
-        else OK((run_gemm<A_KM, B_KN>(c, rem - 1, 2 * prio_cols, L + at(J1 + 1, J0), ld, L + at(J1, J0), ld, K, KR_FULL, TS_NBLK_LE1, epi_store(Kw + at(J1 + 1, J1), ld, false, -1.0, 1.0))));
+        OK((run_gemm<A_KM, B_KN>(c, rem - 1, 2 * prio_cols, L + at(J1 + 1, J0), ld, L + at(J1, J0), ld, K, KR_FULL, TS_NBLK_LE1, epi_store(Kw + at(J1 + 1, J1), ld, false, -1.0, 1.0))));
       }
-      CU(cudaEventRecord(c->ev_prio[0], ss));
+      CU(cudaEventRecord(c->ev_prio, ss));
       prio_pending = true;
     }
     if (rem2 > 0) {
       StreamSwap sw(c, st);
       CU(cudaStreamWaitEvent(st, c->ev_side, 0));  // recorded after side(J1-1); the side stream's later work is not waited for
-      if (rem2 >= t4)
-        OK((run_gemm<A_KM, B_KN>(c, rem2, 2 * rem2, L + at(J2, J0), ld, L + at(J2, J0), ld, K, KR_FULL, TS_NBLK_LE, epi_store(Kw + at(J2, J2), ld, false, -1.0, 1.0))));
-      else
-      OK((run_gemm<A_KM, B_KN, 2>(c, rem2, 2 * rem2, L + at(J2, J0), ld, L + at(J2, J0), ld, K, KR_FULL, TS_NBLK_LE, epi_store(Kw + at(J2, J2), ld, false, -1.0, 1.0))));
+      OK((run_gemm<A_KM, B_KN>(c, rem2, 2 * rem2, L + at(J2, J0), ld, L + at(J2, J0), ld, K, KR_FULL, TS_NBLK_LE, epi_store(Kw + at(J2, J2), ld, false, -1.0, 1.0))));
       CU(cudaEventRecord(c->ev_trail, st));
       trail_pending = true;
     } else {
@@ -1201,7 +1074,7 @@ static int32_t resolve_params(const agp_svgp_params* p, SvgpState& st) {
   OK(fill_kernel_params(&p->kernel, p->D, p->M, st.kp));
   if (p->compute_dtype < AGP_COMPUTE_F64 || p->compute_dtype > AGP_COMPUTE_F64_EMU) return fail(AGP_ERR_INVALID, "unknown compute_dtype %d", p->compute_dtype);
   st.f32 = p->compute_dtype == AGP_COMPUTE_F32 || p->compute_dtype == AGP_COMPUTE_F32_TC_SOLVE;
-  st.f64_emu = p->compute_dtype == AGP_COMPUTE_F64_EMU || f64_s6_i8();
+  st.f64_emu = p->compute_dtype == AGP_COMPUTE_F64_EMU;
   st.f32_tc_solve = p->compute_dtype == AGP_COMPUTE_F32_TC_SOLVE;
   st.lp.kind = p->lik.kind;
   st.lp.sigma2 = p->lik.sigma2;
@@ -1269,20 +1142,9 @@ static int32_t prepare_f32_operands(agp_ctx* c) {
   // Linv itself (rows l, k = l' contiguous) as seven slice planes: the B operand of the INT8 forward solve (f32sweep.cuh EpiE1)
   OK(c->qLi7.ensure((i8e::S * MM + 7) / 8));
   OK(c->sLi7.ensure(Mp));
-  static const bool i8_rn = getenv("AGP_I8_RN") && atoi(getenv("AGP_I8_RN")) != 0;  // experiment: round-to-nearest slices for the forward solve's operands
-  if (i8_rn) i8e::slice_rows_kernel<i8e::S, true><<<(Mp + 7) / 8, 256, 0, c->stream>>>(c->W1.p, Mp, Mp, Mp, reinterpret_cast<signed char*>(c->qLi7.p), Mp, MM, c->sLi7.p);
-  else
   i8e::slice_rows_kernel<i8e::S><<<(Mp + 7) / 8, 256, 0, c->stream>>>(c->W1.p, Mp, Mp, Mp, reinterpret_cast<signed char*>(c->qLi7.p), Mp, MM, c->sLi7.p);
   LAUNCHED(c);
   KCHECK();
-  if (getenv("AGP_DEBUG_LINV")) {  // development aid: the largest entry of the explicit inverse (what the fixed-point slices are relative to)
-    std::vector<double> h(Mp);
-    CU(cudaMemcpyAsync(h.data(), c->sLi7.p, sizeof(double) * Mp, cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaStreamSynchronize(c->stream));
-    double mx = 0.0;
-    for (int i = 0; i < st.M; i++) mx = std::max(mx, h[i]);
-    fprintf(stderr, "[agp] M = %d: pow2 bound of max |Linv| = %.3g\n", st.M, mx);
-  }
   OK(transpose(c, c->W1.p, c->W2.p, Mp, Mp));
   OK(split(c->W2.p, c->fLi));
   // ... and as four INT8 slice planes per row j with a power-of-two row scale: the B operand of the INT8 S5 (f32sweep.cuh EpiE5)
@@ -1293,17 +1155,6 @@ static int32_t prepare_f32_operands(agp_ctx* c) {
   KCHECK();
   return AGP_OK;
 }
-// Float32 mode's reverse-pass solve: "i8" (default) = 4-slice INT8 product with the explicit inverse; "fp64" = the FP64 DMMA triangular solve
-// Float32 mode's forward solve: "i8" (default) = 7-slice (FP64-accurate) INT8 product with the explicit inverse; "fp64" = the DMMA triangular solve
-static bool f32_s1_i8() {
-  static const bool off = getenv("AGP_F32_S1") && strcmp(getenv("AGP_F32_S1"), "fp64") == 0;  // tuning knob
-  return !off;
-}
-static bool f32_s5_i8() {
-  static const bool off = getenv("AGP_F32_S5") && strcmp(getenv("AGP_F32_S5"), "fp64") == 0;  // tuning knob
-  return !off;
-}
-
 // Uploads the parameters and builds every once-per-step operand: zs, zn, Kuu, Lk, Lt, Ut, mt, Bt.
 static int32_t prepare_step(agp_ctx* c, const agp_svgp_params* p) {
   SvgpState& st = c->st;
@@ -1390,10 +1241,7 @@ static int32_t prepare_step(agp_ctx* c, const agp_svgp_params* p) {
     OK(launch_trsm<TR_RHS_FWD>(c, a, Mp / BN));
     OK(transpose(c, c->Bt_rm.p, c->Bt_cm.p, Mp, Mp));
   }
-  {
-    static const bool f64_s1_i8 = getenv("AGP_F64_S1") && strcmp(getenv("AGP_F64_S1"), "i8") == 0;
-    if (st.f32 || (f64_s1_i8 && Mp >= 768)) OK(prepare_f32_operands(c));
-  }
+  if (st.f32) OK(prepare_f32_operands(c));
   st.valid = true;
   return AGP_OK;
 }
@@ -1443,10 +1291,9 @@ struct RedLayout {
 
 // Points per launch group.  Larger chunks amortise launch gaps and wave tails (measured at C4: 2 waves 1988 ms/step,
 // 4 waves 1961, 8 waves 1948); the four M x chunk scratch matrices are capped at ~8 GB.
-// S7 from stored kernel values: plain stationary kinds, split S1 (AGP_KGRAD_FAST=0 restores the recomputing kernel for A/B measurements)
+// S7 from stored kernel values: plain stationary kinds, split S1
 static bool kgrad_fast(const SvgpState& st) {
-  static const bool off = getenv("AGP_KGRAD_FAST") && atoi(getenv("AGP_KGRAD_FAST")) == 0;  // tuning knob
-  return !off && !s1_fused() && st.kp.kind >= AGP_KERNEL_SE && st.kp.kind <= AGP_KERNEL_MATERN52;
+  return !s1_fused() && st.kp.kind >= AGP_KERNEL_SE && st.kp.kind <= AGP_KERNEL_MATERN52;
 }
 static int64_t pick_chunk_cols(agp_ctx* c, int64_t count) {
   const int64_t wave = (int64_t)c->sms * 2 * BN;  // one full wave of column tiles at 2 CTAs / SM
@@ -1481,14 +1328,11 @@ static int32_t ensure_sweep_workspace(agp_ctx* c, int64_t cols, bool grad) {
       OK(c->sAb.ensure(2 * cc));  // scales | column maxima
     }
   }
-  {
-    static const bool f64_s1_i8 = getenv("AGP_F64_S1") && strcmp(getenv("AGP_F64_S1"), "i8") == 0;
-    if ((st.f32 || f64_s1_i8) && f32_s1_i8() && Mp >= 768) {
-      OK(c->Kf.ensure((int64_t)Mp * cc));
-      OK(c->qK.ensure(((int64_t)i8e::S * Mp * cc + 7) / 8));
-      OK(c->sK.ensure(cc));
-      OK(c->sxx_part.ensure((int64_t)2 * (Mp / 32) * cc));  // saa partials | sam partials, one per 32 inducing rows
-    }
+  if (st.f32 && Mp >= 768) {
+    OK(c->Kf.ensure((int64_t)Mp * cc));
+    OK(c->qK.ensure(((int64_t)i8e::S * Mp * cc + 7) / 8));
+    OK(c->sK.ensure(cc));
+    OK(c->sxx_part.ensure((int64_t)2 * (Mp / 32) * cc));  // saa partials | sam partials, one per 32 inducing rows
   }
   if (grad) {
     OK(c->Ab.ensure((int64_t)Mp * cc));
@@ -1505,7 +1349,6 @@ static int32_t ensure_sweep_workspace(agp_ctx* c, int64_t cols, bool grad) {
     const int by_waves = (8 * 2 * c->sms + ntiles - 1) / ntiles;
     const int by_mem = (int)std::max<int64_t>(1, ((int64_t)512 << 20) / (MM * 8));
     c->nsplit = std::max(1, std::min(std::min(by_waves, by_mem), 32));
-    if (const char* e = getenv("AGP_SYRK_SPLIT")) c->nsplit = std::max(1, atoi(e));  // tuning knob
     if (st.f64_emu && !st.f32) c->nsplit = std::max<int>(c->nsplit, (int)((round_up(cc, 128) + 16383) / 16384));  // one slab of G per 16384 points
     OK(c->Gpart.ensure((int64_t)c->nsplit * MM));
     c->nslab = (int)std::max<int64_t>((cc + 2047) / 2048, (Mp + 2047) / 2048);
@@ -1638,7 +1481,7 @@ static int32_t sweep_points(agp_ctx* c, const double* X, const double* y, int64_
       OK(fill(c, c->kpart.p, (int64_t)c->nslab * Mp * kgrad_stride(D), 0.0));
     }
   }
-  const bool emu_s2 = st.f64_emu && !st.f32 && f64_emu_s2() && Mp >= 768;
+  const bool emu_s2 = st.f64_emu && !st.f32 && Mp >= 768;
   if (emu_s2) {  // slices of the rows of Bt^T (columns of Bt, contiguous in the column-major copy), one scale per column
     OK(c->qBt7.ensure(((int64_t)i8e::S * MM + 7) / 8));
     OK(c->sBt7.ensure(Mp));
@@ -1648,8 +1491,7 @@ static int32_t sweep_points(agp_ctx* c, const double* X, const double* y, int64_
   }
   for (int64_t lo = 0; lo < count; lo += cols) {
     const int npts = (int)std::min<int64_t>(cols, count - lo);
-    static const bool f64_i8_exp = getenv("AGP_F64_S1") && strcmp(getenv("AGP_F64_S1"), "i8") == 0;
-    const int ncols = (int)round_up(npts, (st.f32 || f64_i8_exp || st.f64_emu) ? 2 * BN : BN);  // Float32 mode: the tcgen05 stages tile the points by 128
+    const int ncols = (int)round_up(npts, (st.f32 || st.f64_emu) ? 2 * BN : BN);  // Float32 mode: the tcgen05 stages tile the points by 128
     const int tiles_n = ncols / BN;
     const double* pts = X + lo * D;
     // S1: A = Lk^-1 Kuf
@@ -1666,9 +1508,8 @@ static int32_t sweep_points(agp_ctx* c, const double* X, const double* y, int64_
     t1.saa = c->saa.p;
     t1.sam = c->sam.p;
     t1.kp = st.kp;
-    static const bool f64_s1_i8 = getenv("AGP_F64_S1") && strcmp(getenv("AGP_F64_S1"), "i8") == 0;  // experiment: the same solve in the Float64 mode
-    bool a_planes_done = false;
-    if ((st.f32 || f64_s1_i8) && f32_s1_i8() && !s1_fused() && Mp >= 768) {  // (below M ~ 768 the DMMA solve is as fast: C2, M = 512: 11.5 against 12.0 ms)
+    const bool s1_i8 = st.f32 && !s1_fused() && Mp >= 768;
+    if (s1_i8) {  // (below M ~ 768 the DMMA solve is as fast: C2, M = 512: 11.5 against 12.0 ms)
       // Float32 mode: A = Linv Kuf as an FP64-accurate INT8-slice product (i8emu.cuh, 7 slices): generator -> Kf (FP64, also S7's input),
       // point-major slices with exact per-point scales, 28 exact slice products, column sums in the epilogue
       ProfScope ps(c, PC_TRSM_FWD);
@@ -1676,9 +1517,6 @@ static int32_t sweep_points(agp_ctx* c, const double* X, const double* y, int64_
       OK(launch_s1(c, t1, tiles_n, true, true));
       signed char* qK = reinterpret_cast<signed char*>(c->qK.p);
       const int64_t pbytes = (int64_t)Mp * ldc, MM8 = (int64_t)Mp * Mp;
-      static const bool i8_rn = getenv("AGP_I8_RN") && atoi(getenv("AGP_I8_RN")) != 0;
-      if (i8_rn) i8e::transpose_slice_kernel<i8e::S, true><<<(ncols + 31) / 32, 256, 0, c->stream>>>(c->Kf.p, ldc, Mp, ncols, qK, Mp, pbytes, c->sK.p);
-      else
       i8e::transpose_slice_kernel<i8e::S><<<(ncols + 31) / 32, 256, 0, c->stream>>>(c->Kf.p, ldc, Mp, ncols, qK, Mp, pbytes, c->sK.p);
       LAUNCHED(c);
       KCHECK();
@@ -1688,12 +1526,10 @@ static int32_t sweep_points(agp_ctx* c, const double* X, const double* y, int64_
         return fail(AGP_ERR_CUDA, "cuTensorMapEncodeTiled failed");
       const int nparts = Mp / 32;
       i8e::EpiE1 e1{c->A.p, ldc, c->sK.p, c->sLi7.p, c->mt.p, c->sxx_part.p, c->sxx_part.p + (int64_t)nparts * ldc, ldc};
-      if (st.f32) {  // the TF32 planes of A come straight from this epilogue
-        e1.Ah = reinterpret_cast<float*>(c->fA.p);
-        e1.Al = e1.Ah + (int64_t)Mp * ldc;
-        e1.ldf = Mp;
-        a_planes_done = true;
-      }
+      // the TF32 planes of A come straight from this epilogue
+      e1.Ah = reinterpret_cast<float*>(c->fA.p);
+      e1.Al = e1.Ah + (int64_t)Mp * ldc;
+      e1.ldf = Mp;
       i8e::Args g8{Mp, i8e::KM_UPTO_N, 0, 0};
       OK((ensure_smem<i8e::i8emu_gemm_kernel<i8e::EpiE1>>(c, i8e::SMEM_BYTES)));
       i8e::i8emu_gemm_kernel<i8e::EpiE1><<<dim3(Mp / i8e::EN, ncols / i8e::EM, 1), i8e::E_THREADS, i8e::SMEM_BYTES, c->stream>>>(ma, mb, g8, e1);
@@ -1715,7 +1551,7 @@ static int32_t sweep_points(agp_ctx* c, const double* X, const double* y, int64_
     const int64_t MMf = (int64_t)Mp * Mp;
     const dim3 grid5(ncols / t5::TM, Mp / t5::TN, 1);
     if (st.f32) {
-      if (!a_planes_done) {
+      if (!s1_i8) {
         ProfScope ps(c, PC_F32_AUX);
         t5::transpose_split_kernel<<<dim3(ncols / 32, Mp / 32), 256, 0, c->stream>>>(c->A.p, ldc, Mp, ncols, fA, fA + plane, Mp);
         LAUNCHED(c);
@@ -1800,10 +1636,9 @@ static int32_t sweep_points(agp_ctx* c, const double* X, const double* y, int64_
           OK((launch_t5<false, false>(c, grid5, fC, plane, Mp, ncols, reinterpret_cast<float*>(c->fBtr.p), MMf, Mp, Mp, g, e4)));
         } else {
           t5::EpiF4<false> e4{fA, fA + plane, fAb, fAb + plane, fAs, fAs + plane, Mp, c->dmu.p, c->dv.p, c->mt.p, c->Ab.p, ldc};
-          if (f32_s5_i8()) {  // the column maxima of Ab ride along: the INT8 S5 slices without a pass of its own for them
-            CU(cudaMemsetAsync(c->sAb.p + ldc, 0, sizeof(double) * ncols, c->stream));
-            e4.abmax = c->sAb.p + ldc;
-          }
+          // the column maxima of Ab ride along: the INT8 S5 slices without a pass of its own for them
+          CU(cudaMemsetAsync(c->sAb.p + ldc, 0, sizeof(double) * ncols, c->stream));
+          e4.abmax = c->sAb.p + ldc;
           OK((launch_t5<false, false>(c, grid5, fC, plane, Mp, ncols, reinterpret_cast<float*>(c->fBtr.p), MMf, Mp, Mp, g, e4)));
         }
       }
@@ -1812,7 +1647,7 @@ static int32_t sweep_points(agp_ctx* c, const double* X, const double* y, int64_
         t5::EpiF5 e5{c->Ab.p, ldc};
         t5::Args g{Mp, t5::KM_FROM_N, 0, 0, t5::MnDesc()};
         OK((launch_t5<false, false>(c, grid5, fAb, plane, Mp, ncols, reinterpret_cast<float*>(c->fLi.p), MMf, Mp, Mp, g, e5)));
-      } else if (f32_s5_i8()) {
+      } else {
         // Kb = Lk^-T Ab as an exact-accumulation INT8 product with the explicit inverse: Ab (FP64, inducing-major, from the S4 epilogue) is
         // cut into 4 slice planes per point (transpose_slice_kernel), the product overwrites Ab with Kb
         ProfScope ps(c, PC_TRSM_BWD);
@@ -1832,17 +1667,6 @@ static int32_t sweep_points(agp_ctx* c, const double* X, const double* y, int64_
         i8e::i8emu_gemm_kernel<i8e::EpiE5, i8e::S5_NS, i8e::S5_N><<<dim3(Mp / i8e::S5_N, ncols / i8e::EM, 1), i8e::E_THREADS, sm8, c->stream>>>(ma, mb, g8, e5);
         LAUNCHED(c);
         KCHECK();
-      } else {
-        // Kb = Lk^-T Ab stays the FP64 triangular solve, in place on the FP64 inducing-major matrix the S4 epilogue wrote
-        TrsmArgs t5a{};
-        t5a.T = c->Ut.p;
-        t5a.ldt = Mp;
-        t5a.nb = nb;
-        t5a.X = c->Ab.p;
-        t5a.ldx = ldc;
-        t5a.kp = st.kp;
-        ProfScope ps(c, PC_TRSM_BWD);
-        OK(launch_trsm<TR_RHS_BWD>(c, t5a, tiles_n));
       }
       {
         ProfScope ps(c, PC_SYRK);
@@ -2129,9 +1953,6 @@ extern "C" int32_t agp_svgp_finish(agp_ctx* c, double* elbo_out, agp_svgp_grads*
   CU(cudaMemcpyAsync(h_flags, c->d_flags, sizeof h_flags, cudaMemcpyDeviceToHost, c->stream));
   CU(cudaStreamSynchronize(c->stream));
   if (go->dLq) CU(cudaStreamSynchronize(c->stream_copy));
-#if defined(AGP_EXP_NOGEN) || defined(AGP_EXP_NOEXP) || defined(AGP_EXP_WAIT2)
-  h_flags[0] = h_flags[1] = 0;  // timing experiments (tools/s1_experiments.sh) produce garbage on purpose
-#endif
   if (h_scal[SC_PEER_FAILED] != 0.0) return fail(AGP_ERR_NCCL, "%d peer rank(s) failed before the all-reduce; the result is invalid", (int)h_scal[SC_PEER_FAILED]);
   if (h_flags[0] != 0) return fail_not_pd("cov(fz)", h_flags[0]);
   if (h_flags[1] != 0) return fail(AGP_ERR_DOMAIN, "DomainError: a marginal variance is not positive");

@@ -86,82 +86,17 @@ __global__ void cross_k_kernel(double* K, int64_t ld, const double* xs, const do
 // diagonal, a register-resident row solve of the panel and a rank-32 trailing update; then the inverse by the
 // recursive rule  inv([L11 0; L21 L22]) = [X11 0; -X22 L21 X11  X22].
 constexpr int PT_LD = 129;
-constexpr int PT_PLD = 20;  // row pitch of the panel copy read by the DMMA trailing update (20 = 4 mod 16: conflict-free fragments)
 constexpr int PT_SMEM_BYTES = (128 * PT_LD + 64 * 65 + 128) * 8;
 
-// Cholesky of a 32 x 32 diagonal block by one warp, in place in shared memory (lane i owns row i; left-looking: column J is
-// a_iJ - sum_{k<J} l_ik l_Jk, a dot product of the lane's own row with row J, which every lane reads as a broadcast).
-// This warp's per-column dependency chain (shuffle of the diagonal -> rsqrt -> corrections -> store) is the critical path of
-// the whole diagonal-block kernel: tools/pt_timing.cu measures ~14 us per 32-block (~850 cycles per column) for this loop,
-// for a fully unrolled right-looking register version (16 / 10 us cold / warm, ~25 KB of straight-line code) and for a variant
-// with the chain cut to rsqrt + one multiply and the k < J part of the next dot product issued under the rsqrt (14.6 us), so
-// the compact loop is kept (profiles/r03_pt_timing.txt).
-__device__ __forceinline__ void pt_potrf32(double* blk, int lane, double* rdiag, int col0, int* info) {
-  double* row = blk + lane * PT_LD;
-  for (int J = 0; J < 32; J++) {
-    const double* rJ = blk + J * PT_LD;
-    double acc0 = row[J], acc1 = 0.0;
-    int k = 0;
-    for (; k + 1 < J; k += 2) {
-      acc0 = fma(-row[k], rJ[k], acc0);
-      acc1 = fma(-row[k + 1], rJ[k + 1], acc1);
-    }
-    if (k < J) acc0 = fma(-row[k], rJ[k], acc0);
-    const double v = acc0 + acc1;
-    const double d = __shfl_sync(0xffffffffu, v, J);
-    if (lane == 0 && !(d > 0.0)) atomicCAS(info, 0, col0 + J + 1);
-    // sqrt(d), 1/sqrt(d) and v/sqrt(d) from one rsqrt plus FMA corrections (the results agree with sqrt() and the
-    // true quotients to the last bit or one ulp; a dependent sqrt + two divisions cost 4x the latency per column)
-    const double y = rsqrt(d);
-    const double s0 = d * y;
-    const double sq = fma(fma(-s0, s0, d), 0.5 * y, s0);
-    const double inv = fma(fma(-sq, y, 1.0), y, y);
-    const double l0 = v * inv;
-    const double lij = (lane == J) ? sq : fma(fma(-l0, sq, v), inv, l0);
-    if (lane >= J) row[J] = lij;  // rows above the diagonal keep the zero they were loaded with
-    if (lane == J) rdiag[J] = inv;
-    __syncwarp();  // column J is read (as row J's entries) by every later column
-  }
-}
-// The same factorisation with the ROWS IN REGISTERS and a compact loop (round 2, second attempt at the critical path of C3): lane i owns
-// row i as x[k] = A[i][j + k] -- the window slides by one column per step, so that the pivot column is always x[0] and every register
-// index is a compile-time constant although the loop over j is not unrolled (~100 instructions, warm in the instruction cache after the
-// first step, unlike the 10 KB straight-line pt_potrf16).  Right-looking: after column j is scaled, x[k-1] <- x[k] - l_ij l_(j+k)j, where
-// l_(j+k)j is lane j+k's own l_ij, fetched with a shuffle whose source LANE is dynamic (allowed) while the source register is fixed.
-// Slots that slide past column 31 and the entries above the diagonal carry unused values.  Same pivot arithmetic as pt_potrf32.
-__device__ __forceinline__ void pt_potrf32r(double* blk, int lane, double* rdiag, int col0, int* info) {
-  double x[32];
-#pragma unroll
-  for (int c = 0; c < 32; c++) x[c] = blk[lane * PT_LD + c];
-#pragma unroll 1
-  for (int j = 0; j < 32; j++) {
-    const double v = x[0];
-    const double d = __shfl_sync(0xffffffffu, v, j);
-    if (lane == 0 && !(d > 0.0)) atomicCAS(info, 0, col0 + j + 1);
-    const double y = rsqrt(d);
-    const double s0 = d * y;
-    const double sq = fma(fma(-s0, s0, d), 0.5 * y, s0);
-    const double inv = fma(fma(-sq, y, 1.0), y, y);
-    const double l0 = v * inv;
-    const double lij = (lane == j) ? sq : fma(fma(-l0, sq, v), inv, l0);
-#pragma unroll
-    for (int k = 1; k < 16; k++) x[k - 1] = fma(-lij, __shfl_sync(0xffffffffu, lij, (j + k) & 31), x[k]);
-    if (j < 16) {  // columns j + 16 .. j + 31 exist only in the first half of the sweep
-#pragma unroll
-      for (int k = 16; k < 32; k++) x[k - 1] = fma(-lij, __shfl_sync(0xffffffffu, lij, (j + k) & 31), x[k]);
-    } else {
-      x[15] = 0.0;
-    }
-    if (lane >= j) blk[lane * PT_LD + j] = lij;  // rows above the diagonal keep the zero they were loaded with
-    if (lane == j) rdiag[j] = inv;
-  }
-  __syncwarp();
-}
-// Third form (the default): the sliding window of pt_potrf32r, but the scaled column reaches the other lanes through shared memory: every
-// lane publishes its l_ij in two doubled buffers (one shifted by an element, so that the 31 partners l_(j+1)j .. l_(j+31)j start at a 16-byte
-// aligned address whatever the parity of j) and reads them back as 16 broadcast LDS.128.  tools/potrf32_bench.cu, one warp alone, cycles per
-// column: shared-memory left-looking loop 853, sliding window with 62 SHFL 550, with 31 LDS.64 654, with 16 LDS.128 362; the pivot chain
-// alone (shuffle of the pivot, rsqrt, nine dependent FP64 operations, 31 DFMA) is 313 (profiles/r3b_potrf32_variants.jsonl).
+// Cholesky of a 32 x 32 diagonal block by one warp with the rows in registers: lane i owns row i as x[k] = A[i][j + k], a window that
+// slides by one column per step, so that the pivot column is always x[0] and every register index is a compile-time constant although the
+// loop over j is not unrolled.  Right-looking: after column j is scaled, x[k-1] <- x[k] - l_ij l_(j+k)j.  The scaled column reaches the other
+// lanes through shared memory: every lane publishes its l_ij in two doubled buffers (one shifted by an element, so that the 31 partners
+// l_(j+1)j .. l_(j+31)j start at a 16-byte aligned address whatever the parity of j) and reads them back as 16 broadcast LDS.128.  Slots that
+// slide past column 31 and the entries above the diagonal carry unused values.  This warp's per-column dependency chain is the critical
+// path of the whole diagonal-block kernel.  Measured on one warp alone, cycles per column: shared-memory left-looking loop 853, sliding
+// window with 62 SHFL 550, with 31 LDS.64 654, with 16 LDS.128 (this form) 362; the pivot chain alone (shuffle of the pivot, rsqrt, nine
+// dependent FP64 operations, 31 DFMA) is 313 (profiles/r3b_potrf32_variants.jsonl).  The other forms were removed after that measurement.
 // buf: 128 doubles, 16-byte aligned.
 __device__ __forceinline__ void pt_potrf32w(double* blk, int lane, double* rdiag, int col0, int* info, double* buf) {
   double x[32];
@@ -199,61 +134,6 @@ __device__ __forceinline__ void pt_potrf32w(double* blk, int lane, double* rdiag
     __syncwarp();  // the exchange buffers are rewritten by the next step
   }
 }
-// Cholesky of a 16 x 16 diagonal block by one warp with the ROWS IN REGISTERS (lane i < 16 owns row i; lanes 16..31 mirror them):
-// right-looking and fully unrolled, so that every register index is a compile-time constant.  The columns are kept UNSCALED while the
-// sweep runs (LDL^T style: K[i][k] -= K[i][j] K[k][j] / d_j), so that the per-column dependency chain is: broadcast of the pivot ->
-// reciprocal -> one multiply -> one FMA; the square roots -- rsqrt plus FMA corrections, the results agree with sqrt() and the true
-// quotients to the last bit or one ulp -- are taken for all 16 pivots at once after the sweep, lane j for pivot j, and L[i][j] =
-// K(j)[i][j] / sqrt(d_j) is formed from their broadcasts.  (pt_potrf32's shared-memory dot products cost ~850 cycles per column; the
-// first register version, with the rsqrt inside the chain, 530; tools/pt_timing.cu.)
-__device__ __forceinline__ void pt_potrf16(double* blk, int lane, double* rdiag, int col0, int* info) {
-  const int i = lane & 15;
-  double x[16];
-#pragma unroll
-  for (int c = 0; c < 16; c++) x[c] = blk[i * PT_LD + c];
-  double dmine = 1.0;
-#pragma unroll
-  for (int j = 0; j < 16; j++) {
-    const double d = __shfl_sync(0xffffffffu, x[j], j);
-    if (lane == 0 && !(d > 0.0)) atomicCAS(info, 0, col0 + j + 1);
-    if (i == j) dmine = d;
-    const double f = x[j] * __drcp_rn(d);
-#pragma unroll
-    for (int k = j + 1; k < 16; k++) {
-      const double kkj = __shfl_sync(0xffffffffu, x[j], k);
-      x[k] = fma(-f, kkj, x[k]);
-    }
-  }
-  const double y = rsqrt(dmine);
-  const double s0 = dmine * y;
-  const double sq = fma(fma(-s0, s0, dmine), 0.5 * y, s0);
-  const double inv = fma(fma(-sq, y, 1.0), y, y);
-  if (lane < 16) rdiag[lane] = inv;
-#pragma unroll
-  for (int j = 0; j < 16; j++) {
-    const double sqj = __shfl_sync(0xffffffffu, sq, j), invj = __shfl_sync(0xffffffffu, inv, j);
-    const double v = x[j];
-    const double l0 = v * invj;
-    x[j] = (i == j) ? sqj : fma(fma(-l0, sqj, v), invj, l0);
-  }
-  if (lane < 16) {
-#pragma unroll
-    for (int c = 0; c < 16; c++) blk[i * PT_LD + c] = (c <= i) ? x[c] : 0.0;
-  }
-}
-template <int J>
-struct PtSolveRow16 {  // x L_d^T = a for one row of 16 held in x[]
-  static __device__ __forceinline__ void run(double (&x)[16], const double* Ld, const double* rdiag) {
-    x[J] *= rdiag[J];
-#pragma unroll
-    for (int k = J + 1; k < 16; k++) x[k] = fma(-x[J], Ld[k * PT_LD + J], x[k]);
-    PtSolveRow16<J + 1>::run(x, Ld, rdiag);
-  }
-};
-template <>
-struct PtSolveRow16<16> {
-  static __device__ __forceinline__ void run(double (&)[16], const double*, const double*) {}
-};
 template <int J>
 struct PtSolveRow {  // x L_d^T = a for one row held in x[] (right-looking: x[J] is final, then x[k > J] -= x[J] L[k][J])
   static __device__ __forceinline__ void run(double (&x)[32], const double* Ld, const double* rdiag) {
@@ -363,27 +243,14 @@ __global__ void __launch_bounds__(256) potrf_trinv128_kernel(const double* src, 
   const int nact = min(N, (nvalid + 31) & ~31);  // active leading part (multiple of 32)
   if (tid < N) rdiag[tid] = 1.0;
   __syncthreads();
-  // 32-wide blocks.  -DAGP_PT_B16 selects the round-2 experiment: 16-wide blocks with the register-resident pt_potrf16 and a DMMA trailing
-  // update.  Measured (tools/pt_timing.cu, profiles/r2o_pt_timing.txt): a 16 x 16 block costs 4.5 us in registers whether the rsqrt sits
-  // inside the column chain or not (280 ns per column against 425 ns for pt_potrf32), the kernel alone 88.4 -> 81.6 us, but inside the
+  // 32-wide blocks.  16-wide blocks (a register-resident, fully unrolled 16 x 16 factorisation and a DMMA trailing update) were measured
+  // and removed (profiles/r2o_pt_timing.txt): a 16 x 16 block costs 4.5 us in registers whether the rsqrt sits inside the column chain or
+  // not (280 ns per column against 425 ns for the shared-memory 32-wide loop of the time), the kernel alone 88.4 -> 81.6 us, but inside the
   // factorisation -- where every launch meets a cold instruction cache and the unrolled routine is 10 KB -- C3 went from 14.05 to 14.48 ms
-  // per Newton iteration, so it is not the default.
-#ifdef AGP_PT_B16
-  constexpr int PB = 16;
-#else
+  // per Newton iteration.
   constexpr int PB = 32;
-#endif
   for (int o = 0; o < nact; o += PB) {
-    if (warp == 0) {  // diagonal PB x PB block
-#ifdef AGP_PT_LL
-      if (PB == 32) pt_potrf32(s + o * LD + o, lane, rdiag + o, col0 + o, info);
-#elif defined(AGP_PT_SHFL)
-      if (PB == 32) pt_potrf32r(s + o * LD + o, lane, rdiag + o, col0 + o, info);
-#else
-      if (PB == 32) pt_potrf32w(s + o * LD + o, lane, rdiag + o, col0 + o, info, tb);
-#endif
-      else pt_potrf16(s + o * LD + o, lane, rdiag + o, col0 + o, info);
-    }
+    if (warp == 0) pt_potrf32w(s + o * LD + o, lane, rdiag + o, col0 + o, info, tb);  // diagonal PB x PB block
     __syncthreads();
     if (o == 0) { PT_TICK(1) }
     const int T = nact - o - PB;  // rows below the diagonal block (rows >= nact are identity padding: zero below the diagonal)
@@ -392,39 +259,12 @@ __global__ void __launch_bounds__(256) potrf_trinv128_kernel(const double* src, 
       double x[PB];
 #pragma unroll
       for (int j = 0; j < PB; j++) x[j] = row[j];
-      if constexpr (PB == 32) PtSolveRow<0>::run(reinterpret_cast<double(&)[32]>(x), s + o * LD + o, rdiag + o);
-      else PtSolveRow16<0>::run(reinterpret_cast<double(&)[16]>(x), s + o * LD + o, rdiag + o);
+      PtSolveRow<0>::run(x, s + o * LD + o, rdiag + o);
 #pragma unroll
       for (int j = 0; j < PB; j++) row[j] = x[j];
-      if constexpr (PB == 16) {  // second copy with a row pitch of 20 doubles: conflict-free DMMA fragments for the trailing update
-#pragma unroll
-        for (int j = 0; j < PB; j++) tb[tid * PT_PLD + j] = x[j];
-      }
     }
     __syncthreads();
     if (o == 0) { PT_TICK(2) }
-    if constexpr (PB == 16) {
-      // trailing update on the tensor pipe: A[i][c] -= sum_k P[i][k] P[c][k] as 8 x 8 tiles of four m8n8k4 DMMAs, lower tiles only,
-      // dealt round-robin to the 8 warps
-      const int nT = T / 8, g = lane >> 2, t4 = lane & 3;
-      int cnt = 0;
-      for (int bi = 0; bi < nT; bi++)
-        for (int bj = 0; bj <= bi; bj++, cnt++) {
-          if ((cnt & 7) != warp) continue;
-          double acc2[2] = {0.0, 0.0};
-          const double* pa = tb + (bi * 8 + g) * PT_PLD + t4;
-          const double* pb = tb + (bj * 8 + g) * PT_PLD + t4;
-#pragma unroll
-          for (int ks = 0; ks < 4; ks++) dmma884(acc2, pa[4 * ks], pb[4 * ks]);
-          const int r = bi * 8 + g, c = bj * 8 + 2 * t4;
-          double* dst = s + (o + PB + r) * LD + o + PB + c;
-          if (c <= r) dst[0] -= acc2[0];
-          if (c + 1 <= r) dst[1] -= acc2[1];
-        }
-      __syncthreads();
-      if (o == 0) { PT_TICK(3) }
-      continue;
-    }
     // trailing update of the lower triangle: A[i][c] -= sum_k P[i][k] P[c][k]; a thread owns the 4 x 4 elements
     // (ti + a q, tc + b q) so that neighbouring lanes read neighbouring rows (conflict-free with ld = 129); with ti, tc < q an element with
     // b > a always lies above the diagonal, so only the 10 products with b <= a are formed

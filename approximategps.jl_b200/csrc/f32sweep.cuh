@@ -10,8 +10,8 @@
 //   S6  G[i][j] += sum_n As[n][i] A[n][j]                 (MN-major x MN-major straight from the same planes, split over n)
 //   S5  Kb[n][j] = sum_{i >= j} Ab[n][i] Linv[i][j] with the explicit inverse.  As a 3xTF32 product (AGP_COMPUTE_F32_TC_SOLVE) its error is
 //       amplified by cond(Lk) into dZ / d theta (1.4e-4 at the C4 twin: outside the budget); the default is the same product on the INT8 tensor
-//       path with exact accumulation (i8emu.cuh, 5 slices = 35 bits: EpiE5 below), 2.1x faster than the FP64 DMMA solve it replaces
-//       (AGP_F32_S5=fp64 restores that one).
+//       path with exact accumulation (i8emu.cuh, 5 slices = 35 bits: EpiE5 below), measured 2.1x faster than the FP64 DMMA solve it
+//       replaced (which was then removed from this mode).
 #pragma once
 #include "tf32x3.cuh"
 #include "i8emu.cuh"

@@ -283,7 +283,7 @@ inline bool make_map3(CUtensorMap* map, const signed char* ptr, uint64_t k, uint
 }
 
 // slices of a row-major FP64 matrix [rows][ld] (k contiguous): one warp per row -- row maximum, power-of-two scale, S planes [S][rows][ldk]
-template <int NS = S, bool RN = false>
+template <int NS = S>
 __global__ void __launch_bounds__(256) slice_rows_kernel(const double* __restrict__ in, int64_t ld, int rows, int k, signed char* __restrict__ planes, int64_t ldk,
                                                          int64_t plane_bytes, double* __restrict__ scale) {
   const int row = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
@@ -293,12 +293,11 @@ __global__ void __launch_bounds__(256) slice_rows_kernel(const double* __restric
   for (int c = lane; c < k; c += 32) mx = fmax(mx, fabs(src[c]));
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, o));
-  const double sc = (RN ? 2.0 : 1.0) * pow2_scale(mx), inv = 1.0 / sc;
+  const double sc = pow2_scale(mx), inv = 1.0 / sc;
   if (lane == 0) scale[row] = sc;
   for (int c = lane; c < (int)ldk; c += 32) {
     signed char q[NS];
-    if (RN) slice_rn<NS>(c < k ? src[c] : 0.0, inv, q);
-    else slice_n<NS>(c < k ? src[c] : 0.0, inv, q);
+    slice_n<NS>(c < k ? src[c] : 0.0, inv, q);
 #pragma unroll
     for (int i = 0; i < NS; i++) planes[i * plane_bytes + (int64_t)row * ldk + c] = q[i];
   }
@@ -308,7 +307,7 @@ __global__ void __launch_bounds__(256) slice_rows_kernel(const double* __restric
 // k contiguous, one power-of-two scale per point from the exact column maximum.  One CTA per 32 points: a first pass over the strip for the
 // maxima, a second one (an L2 hit: 32 x rows x 8 bytes) through a 32 x 32 shared-memory tile for the transposed, sliced stores.
 // colmax != nullptr: the column maxima are already known (the producing epilogue tracked them with atomicMax) and the first pass is skipped.
-template <int NS, bool RN = false>
+template <int NS>
 __global__ void __launch_bounds__(256) transpose_slice_kernel(const double* __restrict__ in, int64_t ld, int rows, int cols, signed char* __restrict__ planes,
                                                               int64_t ldk, int64_t plane_bytes, double* __restrict__ scale, const double* __restrict__ colmax = nullptr) {
   __shared__ double tile[32][33];
@@ -328,7 +327,7 @@ __global__ void __launch_bounds__(256) transpose_slice_kernel(const double* __re
   if (ty == 0) {
 #pragma unroll
     for (int j = 1; j < 8; j++) mx = fmax(mx, smx[j][tx]);
-    const double sc = (RN ? 2.0 : 1.0) * pow2_scale(mx);
+    const double sc = pow2_scale(mx);
     if (cok) scale[n0 + tx] = sc;
     sinv[tx] = 1.0 / sc;
   }
@@ -342,10 +341,7 @@ __global__ void __launch_bounds__(256) transpose_slice_kernel(const double* __re
       const double inv = sinv[n];
       signed char q[4][NS];
 #pragma unroll
-      for (int e = 0; e < 4; e++) {
-        if (RN) slice_rn<NS>(tile[r4 + e][n], inv, q[e]);
-        else slice_n<NS>(tile[r4 + e][n], inv, q[e]);
-      }
+      for (int e = 0; e < 4; e++) slice_n<NS>(tile[r4 + e][n], inv, q[e]);
 #pragma unroll
       for (int i = 0; i < NS; i++) {
         const char4 v = make_char4(q[0][i], q[1][i], q[2][i], q[3][i]);

@@ -77,7 +77,7 @@ __device__ __forceinline__ void kappa_and_du(int kind, double u, double c, doubl
 // 13 FP64-pipe instructions against ~25 of the CUDA library routine (which spends the rest on the x > 0 / overflow paths this
 // caller cannot reach).  Used by kuf_gen_kernel, which is bound by the FP64 pipe (8 FMAs of distance + the exponential per element),
 // not by HBM.  Error against mpmath over [-708, 0]: below 1 ulp (exact emulation of this
-// operation sequence, and tests/test_gpu_svgp.py::test_kernel_function_values on the device).  x < -708 (result < 1e-307) returns 0.  -DAGP_NO_FAST_EXP restores exp().
+// operation sequence, and tests/test_gpu_svgp.py::test_kernel_function_values on the device).  x < -708 (result < 1e-307) returns 0.
 __device__ const double c_exp2_tab[64] = {
     0x1.0000000000000p+0, 0x1.02c9a3e778061p+0, 0x1.059b0d3158574p+0, 0x1.0874518759bc8p+0,
     0x1.0b5586cf9890fp+0, 0x1.0e3ec32d3d1a2p+0, 0x1.11301d0125b51p+0, 0x1.1429aaea92de0p+0,
@@ -96,9 +96,6 @@ __device__ const double c_exp2_tab[64] = {
     0x1.d5818dcfba487p+0, 0x1.da9e603db3285p+0, 0x1.dfc97337b9b5fp+0, 0x1.e502ee78b3ff6p+0,
     0x1.ea4afa2a490dap+0, 0x1.efa1bee615a27p+0, 0x1.f50765b6e4540p+0, 0x1.fa7c1819e90d8p+0};
 __device__ __forceinline__ double exp_nonpos(double x) {
-#ifdef AGP_NO_FAST_EXP
-  return exp(x);
-#else
   const double t = fma(x, 0x1.71547652b82fep+6, 0x1.8p52);  // low mantissa bits of t = k = round(64 x / ln2) (two's complement)
   const double kd = t - 0x1.8p52;
   double r = fma(-kd, 0x1.62e42fef00000p-7, x);  // exact: the high part of ln2/64 has 20 trailing zero bits, |k| < 2^17
@@ -113,7 +110,6 @@ __device__ __forceinline__ double exp_nonpos(double x) {
   const double v = fma(tj, p, tj);
   const double res = __hiloint2double(__double2hiint(v) + ((ki >> 6) << 20), __double2loint(v));
   return x < -708.0 ? 0.0 : res;
-#endif
 }
 
 

@@ -80,9 +80,6 @@ struct StepIter {
 template <bool SCALED>
 __device__ __forceinline__ void gen_kuf_tile(double* __restrict__ sB, const double* __restrict__ sZ, const double* __restrict__ xs, int row0,
                                              const KernelParams& kp, int warp, int lane, const double* rowscale, const double* dvec, double (&pkd)[2]) {
-#ifdef AGP_EXP_NOGEN
-  return;  // timing experiment only (tools/s1_experiments.sh): results are garbage
-#endif
   const int g = lane >> 2, t = lane & 3;
   const int D = kp.D, kind = kp.kind, Dq = kuf_dp(D), Sx = Dq + 2;
   const int c0 = warp * 8 + 2 * t;  // this thread's two columns
@@ -115,14 +112,8 @@ __device__ __forceinline__ void gen_kuf_tile(double* __restrict__ sB, const doub
   for (int h = 0; h < 2; h++) {
     const int row = row0 + g + 8 * h;
     const bool valid = row < kp.M;
-    double v0, v1;
-#ifdef AGP_EXP_NOEXP
-    v0 = valid ? kp.variance * u[h][0] : 0.0;  // timing experiment only
-    v1 = valid ? kp.variance * u[h][1] : 0.0;
-#else
-    v0 = valid ? kp.variance * kappa_kp(kp, u[h][0]) : 0.0;
-    v1 = valid ? kp.variance * kappa_kp(kp, u[h][1]) : 0.0;
-#endif
+    double v0 = valid ? kp.variance * kappa_kp(kp, u[h][0]) : 0.0;
+    double v1 = valid ? kp.variance * kappa_kp(kp, u[h][1]) : 0.0;
     if (SCALED) {
       const double dv = dvec[row], rsc = rowscale[row];
       pkd[0] = fma(v0, dv, pkd[0]);
@@ -239,12 +230,8 @@ __global__ void __launch_bounds__(NTHREADS, 2) trsm_kernel(TrsmArgs a) {
   for (int step = 0; step < total; step++) {
     // FWD keeps one stage less in flight: the z slab of stage step+1 must have landed so that its Kuf rows can be
     // generated behind this stage's MMAs (the FP64 work of the generator overlaps the DMMA drain of the warp).
-#ifdef AGP_EXP_WAIT2
-    cp_async_wait<S - 2>();  // timing experiment only: the z slab of the next stage may not have landed
-#else
     if (FWD) cp_async_wait<(S >= 3 ? S - 3 : 0)>();
     else cp_async_wait<S - 2>();
-#endif
     __syncthreads();
     if (step + S - 1 < total) issue((step + S - 1) % S);
     cp_async_commit();
