@@ -109,13 +109,36 @@ static int32_t load_nccl() {
   return AGP_OK;
 }
 
+// The INT8 products of S1 (Float32 mode) and of S2 / S6 (AGP_COMPUTE_F64_EMU) run from M = 768: at M = 512 the DMMA stages are as fast
+// (C2 per step: 11.5 against 12.0 ms for S1, 10.7 against 11.3 ms for S6), while the INT8 S6 takes C4 350 -> 250 ms, C5 minibatch 139 -> 74 ms.
+constexpr int I8_MIN_ROWS = 768;
+// The emulated S2 / S6 run only on launch groups of at least this many points; narrower groups stay on DMMA.
+constexpr int I8_MIN_COLS = 2048;
+
+// Engine of each GEMM-shaped stage of the sweep, fixed per step by compute_dtype and M (resolve_params).
+//   DMMA: the Float64 kernels of sweep.cuh / gemm.cuh (S1: kuf_gen_kernel + blocked TRSM);
+//   TF32: 3xTF32 products on tcgen05 (f32sweep.cuh);  I8: FP64-accurate INT8-slice products on tcgen05 (i8emu.cuh; S5: five slices).
+enum Engine { ENG_DMMA, ENG_TF32, ENG_I8 };
+struct SweepPlan {
+  int pts_tile = BN;  // launch groups are padded to this many points (128 in the tcgen05 modes)
+  Engine s1 = ENG_DMMA, s2 = ENG_DMMA, s4 = ENG_DMMA, s5 = ENG_DMMA, s6 = ENG_DMMA;
+  bool s7_streamed = false;  // S7 reads Kuf and kappa' back from S1 (plain stationary kinds) instead of recomputing them
+  // the plan of one launch group of ncols points
+  SweepPlan at_width(int ncols) const {
+    SweepPlan g = *this;
+    if (ncols < I8_MIN_COLS) {
+      if (g.s2 == ENG_I8) g.s2 = ENG_DMMA;
+      if (g.s6 == ENG_I8) g.s6 = ENG_DMMA;
+    }
+    return g;
+  }
+};
+
 // Everything the sweep needs that depends on one agp_svgp_params (uploaded once per step).
 struct SvgpState {
   bool valid = false;
   bool sweep_pending = false;  // agp_svgp_sweep has filled the reduce buffer and agp_svgp_finish has not consumed it yet
-  bool f32 = false;            // params.compute_dtype != AGP_COMPUTE_F64: S2 / S4 / S6 on the tcgen05 3xTF32 path (f32sweep.cuh)
-  bool f64_emu = false;        // AGP_COMPUTE_F64_EMU: S6 as an FP64-accurate INT8-slice product (i8emu.cuh), everything else as Float64
-  bool f32_tc_solve = false;   // AGP_COMPUTE_F32_TC_SOLVE: the reverse-pass solve S5 as a 3xTF32 product with the explicit inverse as well
+  SweepPlan plan;
   int M = 0, Mp = 0, D = 0, nb = 0;
   int n_scale = 1;
   bool centered = false;
@@ -525,7 +548,7 @@ static int32_t ensure_smem(agp_ctx* c, int bytes) {
 template <int MODE, int S>
 static int32_t launch_trsm_s(agp_ctx* c, const TrsmArgs& a, int tiles_n) {
   using Cfg = StageCfg<A_KM, B_KN>;
-  const int Sx = (MODE == TR_KUF_FWD || MODE == TR_KUF_FWD_SCALED) ? kuf_dp(a.kp.D) + 2 : 0;
+  const int Sx = MODE == TR_KUF_FWD_SCALED ? kuf_dp(a.kp.D) + 2 : 0;
   const int smem = (S * (Cfg::elems + BK * Sx) + 64 * Sx) * 8 + 16;
   OK((ensure_smem<trsm_kernel<MODE, S>>(c, smem)));
   trsm_kernel<MODE, S><<<tiles_n, NTHREADS, smem, c->stream>>>(a);
@@ -534,20 +557,20 @@ static int32_t launch_trsm_s(agp_ctx* c, const TrsmArgs& a, int tiles_n) {
   return AGP_OK;
 }
 // 4 pipeline stages; the Kuf generator drops to 3 when the z slabs of a wide input (D > 8) would cost the second CTA per SM
-// S1 = cov(f.prior, z, x) + the forward solve (SVA.jl:216-217).  Default: kuf_gen_kernel writes the Kuf tile of the launch group into X
-// and the solve runs in place on it (TR_RHS_FWD_SUMS); AGP_S1_FUSED=1 selects the round-1 kernel that generates Kuf inside the DMMA
-// pipeline instead (kept for A/B measurements and used by the Laplace prediction path in its SCALED form).
 template <int MODE>
-static int32_t launch_trsm(agp_ctx* c, const TrsmArgs& a, int tiles_n);
-static bool s1_fused() {
-  static const bool fused = getenv("AGP_S1_FUSED") && atoi(getenv("AGP_S1_FUSED")) != 0;  // tuning knob
-  return fused;
+static int32_t launch_trsm(agp_ctx* c, const TrsmArgs& a, int tiles_n) {
+  if constexpr (MODE == TR_KUF_FWD_SCALED) {
+    if (a.kp.D > 8) return launch_trsm_s<MODE, 3>(c, a, tiles_n);
+  }
+  return launch_trsm_s<MODE, 4>(c, a, tiles_n);
 }
+
+// S1 = cov(f.prior, z, x) + the forward solve (SVA.jl:216-217): kuf_gen_kernel writes the Kuf tile of the launch group into X and the
+// solve runs in place on it (TR_RHS_FWD_SUMS), with the column sums a^T a and a^T mt.
 // keep = true (reverse pass of a stationary kernel): Kuf goes to c->Kf and variance * kappa'(u) to c->DKb, the solve reads Kf and writes
 // t1.X; S7 then contracts the cotangent with the stored values (kgrad_kernel FAST) instead of recomputing distances and exp.
 // gen_only = true: only the generator runs (into c->Kf); the caller solves by other means (Float32 mode: INT8 product with the explicit inverse).
 static int32_t launch_s1(agp_ctx* c, const TrsmArgs& t1_in, int tiles_n, bool keep = false, bool gen_only = false) {
-  if (s1_fused() && !gen_only) return launch_trsm<TR_KUF_FWD>(c, t1_in, tiles_n);
   TrsmArgs t1 = t1_in;
   KufGenArgs g{};
   // (SqExponential: kappa' = -kappa / 2, S7 needs only Kuf itself: one matrix written here instead of two)
@@ -584,10 +607,17 @@ static int32_t launch_s1(agp_ctx* c, const TrsmArgs& t1_in, int tiles_n, bool ke
   return launch_trsm<TR_RHS_FWD_SUMS>(c, t1, tiles_n);
 }
 
+// X <- Lk^-1 X (TR_RHS_FWD) or Lk^-T X (TR_RHS_BWD) in place; X row-major [Mp][ldx], tiles_n tiles of 64 columns
 template <int MODE>
-static int32_t launch_trsm(agp_ctx* c, const TrsmArgs& a, int tiles_n) {
-  if ((MODE == TR_KUF_FWD || MODE == TR_KUF_FWD_SCALED) && a.kp.D > 8) return launch_trsm_s<MODE, 3>(c, a, tiles_n);
-  return launch_trsm_s<MODE, 4>(c, a, tiles_n);
+static int32_t solve_lk(agp_ctx* c, double* X, int64_t ldx, int tiles_n) {
+  TrsmArgs a{};
+  a.T = MODE == TR_RHS_BWD ? c->Ut.p : c->Lt.p;
+  a.ldt = c->st.Mp;
+  a.nb = c->st.nb;
+  a.X = X;
+  a.ldx = ldx;
+  a.kp = c->st.kp;
+  return launch_trsm<MODE>(c, a, tiles_n);
 }
 
 template <int LA, int LB, int S = StageCfg<LA, LB>::stages, class Epi>
@@ -1073,9 +1103,17 @@ static int32_t resolve_params(const agp_svgp_params* p, SvgpState& st) {
   st.jitter = p->jitter;
   OK(fill_kernel_params(&p->kernel, p->D, p->M, st.kp));
   if (p->compute_dtype < AGP_COMPUTE_F64 || p->compute_dtype > AGP_COMPUTE_F64_EMU) return fail(AGP_ERR_INVALID, "unknown compute_dtype %d", p->compute_dtype);
-  st.f32 = p->compute_dtype == AGP_COMPUTE_F32 || p->compute_dtype == AGP_COMPUTE_F32_TC_SOLVE;
-  st.f64_emu = p->compute_dtype == AGP_COMPUTE_F64_EMU;
-  st.f32_tc_solve = p->compute_dtype == AGP_COMPUTE_F32_TC_SOLVE;
+  SweepPlan& pl = st.plan;
+  pl = SweepPlan{};
+  if (p->compute_dtype != AGP_COMPUTE_F64) pl.pts_tile = 2 * BN;
+  if (p->compute_dtype == AGP_COMPUTE_F32 || p->compute_dtype == AGP_COMPUTE_F32_TC_SOLVE) {
+    pl.s1 = st.Mp >= I8_MIN_ROWS ? ENG_I8 : ENG_DMMA;
+    pl.s2 = pl.s4 = pl.s6 = ENG_TF32;
+    pl.s5 = p->compute_dtype == AGP_COMPUTE_F32_TC_SOLVE ? ENG_TF32 : ENG_I8;
+  } else if (p->compute_dtype == AGP_COMPUTE_F64_EMU && st.Mp >= I8_MIN_ROWS) {
+    pl.s2 = pl.s6 = ENG_I8;
+  }
+  pl.s7_streamed = st.kp.kind >= AGP_KERNEL_SE && st.kp.kind <= AGP_KERNEL_MATERN52;
   st.lp.kind = p->lik.kind;
   st.lp.sigma2 = p->lik.sigma2;
   int method = p->expect.method;
@@ -1109,8 +1147,7 @@ static int32_t resolve_params(const agp_svgp_params* p, SvgpState& st) {
 // S2, row-major memory = the [i][j] operand of S4) and the explicit inverse Linv = Lk^-1 (a block TRSM on the identity, as the Laplace
 // pullback builds B^-1), transposed to the [j][i] operand of S5.
 static int32_t prepare_f32_operands(agp_ctx* c) {
-  SvgpState& st = c->st;
-  const int Mp = st.Mp, nb = st.nb;
+  const int Mp = c->st.Mp;
   const int64_t MM = (int64_t)Mp * Mp;
   if (!t5::encode_tiled_fn()) return fail(AGP_ERR_CUDA, "cuTensorMapEncodeTiled is not available from this driver (Float32 mode needs TMA tensor maps)");
   DevBuf* planes[] = {&c->fBtc, &c->fBtr, &c->fLi};
@@ -1131,14 +1168,7 @@ static int32_t prepare_f32_operands(agp_ctx* c) {
   set_diag_kernel<<<(Mp + 255) / 256, 256, 0, c->stream>>>(c->W1.p, Mp, Mp, 1.0);
   LAUNCHED(c);
   KCHECK();
-  TrsmArgs a{};
-  a.T = c->Lt.p;
-  a.ldt = Mp;
-  a.nb = nb;
-  a.X = c->W1.p;
-  a.ldx = Mp;
-  a.kp = st.kp;
-  OK(launch_trsm<TR_RHS_FWD>(c, a, Mp / BN));
+  OK(solve_lk<TR_RHS_FWD>(c, c->W1.p, Mp, Mp / BN));
   // Linv itself (rows l, k = l' contiguous) as seven slice planes: the B operand of the INT8 forward solve (f32sweep.cuh EpiE1)
   OK(c->qLi7.ensure((i8e::S * MM + 7) / 8));
   OK(c->sLi7.ensure(Mp));
@@ -1224,24 +1254,15 @@ static int32_t prepare_step(agp_ctx* c, const agp_svgp_params* p) {
     vec_to_rhs_kernel<<<(Mp * 64 + 255) / 256, 256, 0, c->stream>>>(c->mvec.p, st.mean_const, M, Mp, c->vec64.p);
     LAUNCHED(c);
     KCHECK();
-    TrsmArgs a{};
-    a.T = c->Lt.p;
-    a.ldt = Mp;
-    a.nb = nb;
-    a.X = c->vec64.p;
-    a.ldx = 64;
-    a.kp = st.kp;
-    OK(launch_trsm<TR_RHS_FWD>(c, a, 1));
+    OK(solve_lk<TR_RHS_FWD>(c, c->vec64.p, 64, 1));
     rhs_to_vec_kernel<<<(Mp + 255) / 256, 256, 0, c->stream>>>(c->vec64.p, Mp, c->mt.p);
     LAUNCHED(c);
     KCHECK();
     OK(transpose(c, c->Lq.p, c->Bt_rm.p, Mp, Mp));  // row-major Lq as the right-hand side
-    a.X = c->Bt_rm.p;
-    a.ldx = Mp;
-    OK(launch_trsm<TR_RHS_FWD>(c, a, Mp / BN));
+    OK(solve_lk<TR_RHS_FWD>(c, c->Bt_rm.p, Mp, Mp / BN));
     OK(transpose(c, c->Bt_rm.p, c->Bt_cm.p, Mp, Mp));
   }
-  if (st.f32) OK(prepare_f32_operands(c));
+  if (st.plan.s2 == ENG_TF32) OK(prepare_f32_operands(c));  // Float32 mode
   st.valid = true;
   return AGP_OK;
 }
@@ -1291,10 +1312,6 @@ struct RedLayout {
 
 // Points per launch group.  Larger chunks amortise launch gaps and wave tails (measured at C4: 2 waves 1988 ms/step,
 // 4 waves 1961, 8 waves 1948); the four M x chunk scratch matrices are capped at ~8 GB.
-// S7 from stored kernel values: plain stationary kinds, split S1
-static bool kgrad_fast(const SvgpState& st) {
-  return !s1_fused() && st.kp.kind >= AGP_KERNEL_SE && st.kp.kind <= AGP_KERNEL_MATERN52;
-}
 static int64_t pick_chunk_cols(agp_ctx* c, int64_t count) {
   const int64_t wave = (int64_t)c->sms * 2 * BN;  // one full wave of column tiles at 2 CTAs / SM
   const int64_t by_mem = (int64_t)12e9 / (6 * 8 * std::max(c->st.Mp, BM)) / wave;  // six M x chunk scratch matrices
@@ -1305,6 +1322,7 @@ static int64_t pick_chunk_cols(agp_ctx* c, int64_t count) {
 
 static int32_t ensure_sweep_workspace(agp_ctx* c, int64_t cols, bool grad) {
   const SvgpState& st = c->st;
+  const SweepPlan& pl = st.plan;
   const int Mp = st.Mp, D = st.D, nb = st.nb;
   const int64_t MM = (int64_t)Mp * Mp;
   if (cols > c->chunk_cols) c->chunk_cols = cols;
@@ -1313,23 +1331,28 @@ static int32_t ensure_sweep_workspace(agp_ctx* c, int64_t cols, bool grad) {
   OK(c->C.ensure((int64_t)Mp * cc));
   OK(c->saa.ensure(cc));
   OK(c->sam.ensure(cc));
-  OK(c->scc_part.ensure((int64_t)(st.f64_emu ? 4 : 2) * nb * cc));  // (Float32 mode: one partial per 64-column half of a 128-column tile; emulated S2: one per 32 rows)
+  OK(c->scc_part.ensure((int64_t)(pl.s2 == ENG_I8 ? 4 : 2) * nb * cc));  // column-sum partials of S2 (sweep_s3)
   OK(c->dmu.ensure(cc));
   OK(c->dv.ensure(cc));
   OK(c->sc_part.ensure((cc / 256 + 2) * NSC));
   OK(c->red.ensure(RedLayout(Mp, D).total));
-  if (st.f32) {
+  if (pl.s2 == ENG_TF32) {
     OK(c->fA.ensure((int64_t)Mp * cc));
     OK(c->fC.ensure((int64_t)Mp * cc));
-    if (grad) {
-      OK(c->fAb.ensure((int64_t)Mp * cc));
-      OK(c->fAs.ensure((int64_t)Mp * cc));
-      OK(c->qAb.ensure(((int64_t)i8e::S5_NS * Mp * cc + 7) / 8));
-      OK(c->sAb.ensure(2 * cc));  // scales | column maxima
-    }
   }
-  if (st.f32 && Mp >= 768) {
+  if (grad && pl.s4 == ENG_TF32) {
+    OK(c->fAb.ensure((int64_t)Mp * cc));
+    OK(c->fAs.ensure((int64_t)Mp * cc));
+  }
+  if (grad && pl.s5 == ENG_I8) {
+    OK(c->qAb.ensure(((int64_t)i8e::S5_NS * Mp * cc + 7) / 8));
+    OK(c->sAb.ensure(2 * cc));  // scales | column maxima
+  }
+  if (pl.s1 == ENG_I8 || (grad && pl.s7_streamed)) {  // S1 keeps Kuf (and kappa' for the Matern kinds): the INT8 S1 solves from it, S7 reads it
     OK(c->Kf.ensure((int64_t)Mp * cc));
+    if (st.kp.kind != AGP_KERNEL_SE) OK(c->DKb.ensure((int64_t)Mp * cc));
+  }
+  if (pl.s1 == ENG_I8) {
     OK(c->qK.ensure(((int64_t)i8e::S * Mp * cc + 7) / 8));
     OK(c->sK.ensure(cc));
     OK(c->sxx_part.ensure((int64_t)2 * (Mp / 32) * cc));  // saa partials | sam partials, one per 32 inducing rows
@@ -1337,10 +1360,6 @@ static int32_t ensure_sweep_workspace(agp_ctx* c, int64_t cols, bool grad) {
   if (grad) {
     OK(c->Ab.ensure((int64_t)Mp * cc));
     OK(c->As.ensure((int64_t)Mp * cc));
-    if (kgrad_fast(st)) {
-      OK(c->Kf.ensure((int64_t)Mp * cc));
-      if (st.kp.kind != AGP_KERNEL_SE) OK(c->DKb.ensure((int64_t)Mp * cc));
-    }
     OK(c->gpart.ensure((cc / BN) * Mp));
     const int ntiles = nb * (nb + 1);
     // K-splits of the SYRK: about eight waves of CTAs so that the cheap diagonal tiles (3/8 and 7/8 of a full tile's MMAs)
@@ -1349,7 +1368,7 @@ static int32_t ensure_sweep_workspace(agp_ctx* c, int64_t cols, bool grad) {
     const int by_waves = (8 * 2 * c->sms + ntiles - 1) / ntiles;
     const int by_mem = (int)std::max<int64_t>(1, ((int64_t)512 << 20) / (MM * 8));
     c->nsplit = std::max(1, std::min(std::min(by_waves, by_mem), 32));
-    if (st.f64_emu && !st.f32) c->nsplit = std::max<int>(c->nsplit, (int)((round_up(cc, 128) + 16383) / 16384));  // one slab of G per 16384 points
+    if (pl.s6 == ENG_I8) c->nsplit = std::max<int>(c->nsplit, (int)((round_up(cc, 128) + 16383) / 16384));  // one slab of G per 16384 points
     OK(c->Gpart.ensure((int64_t)c->nsplit * MM));
     c->nslab = (int)std::max<int64_t>((cc + 2047) / 2048, (Mp + 2047) / 2048);
     OK(c->kpart.ensure((int64_t)c->nslab * Mp * kgrad_stride(D)));
@@ -1463,11 +1482,316 @@ static int32_t launch_t5(agp_ctx* c, dim3 grid, const float* A, int64_t planeA, 
   return AGP_OK;
 }
 
+// One FP64-accurate INT8-slice product (i8emu.cuh).  Each operand is NS slice planes (plane bytes apart) of [rows][k] int8, k contiguous;
+// A is tiled by EM rows, B by N rows.
+template <class Epi, int NS = i8e::S, int N = i8e::EN>
+static int32_t launch_i8(agp_ctx* c, const DevBuf& A, uint64_t rowsA, int64_t planeA, const DevBuf& B, uint64_t rowsB, int64_t planeB, uint64_t k,
+                         dim3 grid, const i8e::Args& g, const Epi& epi) {
+  CUtensorMap ma, mb;
+  if (!i8e::make_map3(&ma, reinterpret_cast<const signed char*>(A.p), k, rowsA, k, planeA, i8e::EM, NS) ||
+      !i8e::make_map3(&mb, reinterpret_cast<const signed char*>(B.p), k, rowsB, k, planeB, N, NS))
+    return fail(AGP_ERR_CUDA, "cuTensorMapEncodeTiled failed");
+  constexpr int smem = i8e::Cfg<NS, N>::smem_bytes;
+  OK((ensure_smem<i8e::i8emu_gemm_kernel<Epi, NS, N>>(c, smem)));
+  i8e::i8emu_gemm_kernel<Epi, NS, N><<<grid, i8e::E_THREADS, smem, c->stream>>>(ma, mb, g, epi);
+  LAUNCHED(c);
+  KCHECK();
+  return AGP_OK;
+}
+
+// S1's arguments for the points [pts, pts + npts): A = Lk^-1 Kuf into X (row stride ldx), column sums into saa / sam
+static TrsmArgs s1_args(agp_ctx* c, double* X, int64_t ldx, const double* pts, int npts) {
+  TrsmArgs t1{};
+  t1.T = c->Lt.p;
+  t1.ldt = c->st.Mp;
+  t1.nb = c->st.nb;
+  t1.X = X;
+  t1.ldx = ldx;
+  t1.pts = pts;
+  t1.npts = npts;
+  t1.zsp = c->zsp.p;
+  t1.mt = c->mt.p;
+  t1.saa = c->saa.p;
+  t1.sam = c->sam.p;
+  t1.kp = c->st.kp;
+  return t1;
+}
+
+// The stages of one launch group of the sweep: npts points at pts, padded to ncols columns of the [Mp][chunk_cols] scratch matrices;
+// pl is the step's plan at that width (SweepPlan::at_width).
+
+// S1: A = Lk^-1 Kuf with the column sums a^T a and a^T mt.  keep: S7 streams Kuf (and kappa') back from S1.
+static int32_t sweep_s1(agp_ctx* c, const SweepPlan& pl, const double* pts, int npts, int ncols, bool keep) {
+  const int Mp = c->st.Mp;
+  const int64_t ldc = c->chunk_cols, plane = (int64_t)Mp * ldc;
+  ProfScope ps(c, PC_TRSM_FWD);
+  switch (pl.s1) {
+    case ENG_I8: {
+      // A = Linv Kuf as an INT8-slice product (7 slices): generator -> Kf (FP64, also S7's input), point-major slices with exact
+      // per-point scales, 28 exact slice products, column sums in the epilogue
+      OK(launch_s1(c, s1_args(c, c->A.p, ldc, pts, npts), ncols / BN, true, true));
+      i8e::transpose_slice_kernel<i8e::S><<<(ncols + 31) / 32, 256, 0, c->stream>>>(c->Kf.p, ldc, Mp, ncols, reinterpret_cast<signed char*>(c->qK.p), Mp,
+                                                                                  plane, c->sK.p);
+      LAUNCHED(c);
+      KCHECK();
+      const int nparts = Mp / 32;
+      i8e::EpiE1 e1{c->A.p, ldc, c->sK.p, c->sLi7.p, c->mt.p, c->sxx_part.p, c->sxx_part.p + (int64_t)nparts * ldc, ldc};
+      // the TF32 planes of A come straight from this epilogue
+      e1.Ah = reinterpret_cast<float*>(c->fA.p);
+      e1.Al = e1.Ah + plane;
+      e1.ldf = Mp;
+      OK((launch_i8<i8e::EpiE1>(c, c->qK, ncols, plane, c->qLi7, Mp, (int64_t)Mp * Mp, Mp, dim3(Mp / i8e::EN, ncols / i8e::EM, 1),
+                                i8e::Args{Mp, i8e::KM_UPTO_N, 0, 0}, e1)));
+      i8e::colsum_reduce_kernel<<<(ncols + 255) / 256, 256, 0, c->stream>>>(c->sxx_part.p, nparts, ldc, ncols, c->saa.p, c->sam.p);
+      LAUNCHED(c);
+      KCHECK();
+      return AGP_OK;
+    }
+    default:
+      return launch_s1(c, s1_args(c, c->A.p, ldc, pts, npts), ncols / BN, keep);
+  }
+}
+
+// S2: C = Bt^T A with partial column sums of c^T c
+static int32_t sweep_s2(agp_ctx* c, const SweepPlan& pl, int ncols) {
+  const int Mp = c->st.Mp;
+  const int64_t ldc = c->chunk_cols, plane = (int64_t)Mp * ldc, MM = (int64_t)Mp * Mp;
+  switch (pl.s2) {
+    case ENG_TF32: {
+      // point-major hi / lo planes of A (unless the INT8 S1 wrote them), then C = A Bt on the tcgen05 path (f32sweep.cuh)
+      float* fA = reinterpret_cast<float*>(c->fA.p);
+      float* fC = reinterpret_cast<float*>(c->fC.p);
+      if (pl.s1 != ENG_I8) {
+        ProfScope ps(c, PC_F32_AUX);
+        t5::transpose_split_kernel<<<dim3(ncols / 32, Mp / 32), 256, 0, c->stream>>>(c->A.p, ldc, Mp, ncols, fA, fA + plane, Mp);
+        LAUNCHED(c);
+        KCHECK();
+      }
+      ProfScope ps(c, PC_GEMM_BTA);
+      t5::EpiF2 e2{fC, fC + plane, Mp, c->scc_part.p, ldc};
+      t5::Args g{Mp, t5::KM_FROM_N, 0, 0, t5::MnDesc()};
+      return launch_t5<false, false>(c, dim3(ncols / t5::TM, Mp / t5::TN, 1), fA, plane, Mp, ncols, reinterpret_cast<float*>(c->fBtc.p), MM, Mp, Mp, g, e2);
+    }
+    case ENG_I8: {
+      // C[n][j] = sum_{l >= j} A[n][l] Bt[l][j].  The point-major slice planes of A live in the buffer that S6 refills with its own
+      // planes later in this launch group.
+      ProfScope ps(c, PC_GEMM_BTA);
+      OK(c->q6As.ensure(((int64_t)i8e::S * plane + 7) / 8));
+      OK(c->sPm.ensure(ldc));
+      i8e::transpose_slice_kernel<i8e::S><<<(ncols + 31) / 32, 256, 0, c->stream>>>(c->A.p, ldc, Mp, ncols, reinterpret_cast<signed char*>(c->q6As.p), Mp,
+                                                                                  plane, c->sPm.p);
+      LAUNCHED(c);
+      KCHECK();
+      i8e::EpiE2 e2{c->C.p, ldc, c->sPm.p, c->sBt7.p, c->scc_part.p, ldc};
+      return launch_i8<i8e::EpiE2>(c, c->q6As, ncols, plane, c->qBt7, Mp, MM, Mp, dim3(Mp / i8e::EN, ncols / i8e::EM, 1), i8e::Args{Mp, i8e::KM_FROM_N, 0, 0}, e2);
+    }
+    default: {
+      // A operand (m=j, k=l) = Bt[l][j] = Bt_rm[l*Mp + j]; nonzero for l >= j
+      EpiS2 e2{c->C.p, ldc, c->scc_part.p, ldc};
+      ProfScope ps(c, PC_GEMM_BTA);
+      return run_gemm<A_KM, B_KN>(c, c->st.nb, ncols / BN, c->Bt_rm.p, Mp, c->A.p, ldc, Mp, KR_UPPER, TS_ALL, e2);
+    }
+  }
+}
+
+// S3: the per-point stage of the points [lo, lo + npts) of X (and y, mu_out, var_out), then (unless predicting) their scalar sums into scal
+static int32_t sweep_s3(agp_ctx* c, const SweepPlan& pl, const double* X, const double* y, int64_t lo, int npts, int ncols, bool predict,
+                        double* mu_out, double* var_out, double* scal) {
+  const SvgpState& st = c->st;
+  PerPointArgs pp{};
+  pp.saa = c->saa.p;
+  pp.sam = c->sam.p;
+  pp.scc_part = c->scc_part.p;
+  pp.ldp = c->chunk_cols;
+  pp.nb = pl.s2 == ENG_TF32 ? 2 * st.nb : pl.s2 == ENG_I8 ? 4 * st.nb : st.nb;  // the column-sum partials S2 wrote
+  pp.pts = X + lo * st.D;
+  pp.y = y ? y + lo : nullptr;
+  pp.npts = npts;
+  pp.ncols = ncols;
+  pp.scale = st.scale;
+  pp.mean_const = st.mean_const;
+  pp.kp = st.kp;
+  pp.lp = st.lp;
+  pp.dmu = c->dmu.p;
+  pp.dv = c->dv.p;
+  pp.mu_out = mu_out ? mu_out + lo : nullptr;
+  pp.var_out = var_out ? var_out + lo : nullptr;
+  pp.sc_part = c->sc_part.p;
+  pp.flag = c->d_flags + 1;
+  pp.predict_only = predict ? 1 : 0;
+  pp.point0 = st.point_base + lo;
+  const int pblocks = (ncols + PP_POINTS_PER_BLOCK - 1) / PP_POINTS_PER_BLOCK;
+  ProfScope ps(c, PC_PERPOINT);
+  perpoint_kernel<<<pblocks, 256, 0, c->stream>>>(pp);
+  LAUNCHED(c);
+  KCHECK();
+  if (predict) return AGP_OK;
+  const int nsc_used = st.kp.kind == AGP_KERNEL_LINEAR ? SC_DS + st.D : SC_DS;
+  scal_reduce_kernel<<<1, 256, 0, c->stream>>>(c->sc_part.p, pblocks, nsc_used, scal);
+  LAUNCHED(c);
+  KCHECK();
+  return AGP_OK;
+}
+
+// S4: Ab = dmu (x) mt + 2 dv (Bt C - A), As = dv A (the DMMA epilogue also accumulates g += A dmu)
+static int32_t sweep_s4(agp_ctx* c, const SweepPlan& pl, int ncols) {
+  const int Mp = c->st.Mp;
+  const int64_t ldc = c->chunk_cols, plane = (int64_t)Mp * ldc, MM = (int64_t)Mp * Mp;
+  ProfScope ps(c, PC_GEMM_BC);
+  switch (pl.s4) {
+    case ENG_TF32: {
+      float* fA = reinterpret_cast<float*>(c->fA.p);
+      float* fC = reinterpret_cast<float*>(c->fC.p);
+      float* fAb = reinterpret_cast<float*>(c->fAb.p);
+      float* fAs = reinterpret_cast<float*>(c->fAs.p);
+      const float* fBtr = reinterpret_cast<float*>(c->fBtr.p);
+      const dim3 grid(ncols / t5::TM, Mp / t5::TN, 1);
+      t5::Args g{Mp, t5::KM_UPTO_N, 0, 0, t5::MnDesc()};
+      if (pl.s5 == ENG_TF32) {
+        t5::EpiF4<true> e4{fA, fA + plane, fAb, fAb + plane, fAs, fAs + plane, Mp, c->dmu.p, c->dv.p, c->mt.p, c->Ab.p, ldc};
+        return launch_t5<false, false>(c, grid, fC, plane, Mp, ncols, fBtr, MM, Mp, Mp, g, e4);
+      }
+      t5::EpiF4<false> e4{fA, fA + plane, fAb, fAb + plane, fAs, fAs + plane, Mp, c->dmu.p, c->dv.p, c->mt.p, c->Ab.p, ldc};
+      // the column maxima of Ab ride along: the INT8 S5 slices without a pass of its own for them
+      CU(cudaMemsetAsync(c->sAb.p + ldc, 0, sizeof(double) * ncols, c->stream));
+      e4.abmax = c->sAb.p + ldc;
+      return launch_t5<false, false>(c, grid, fC, plane, Mp, ncols, fBtr, MM, Mp, Mp, g, e4);
+    }
+    default: {
+      // A operand (m=j,k=l) = Bt[j][l], l <= j
+      EpiS4 e4{c->A.p, c->Ab.p, c->As.p, ldc, c->dmu.p, c->dv.p, c->mt.p, c->gpart.p, Mp};
+      return run_gemm<A_KM, B_KN>(c, c->st.nb, ncols / BN, c->Bt_cm.p, Mp, c->C.p, ldc, Mp, KR_LOWER, TS_ALL, e4);
+    }
+  }
+}
+
+// S5: Kb = Lk^-T Ab, in place
+static int32_t sweep_s5(agp_ctx* c, const SweepPlan& pl, int ncols) {
+  const int Mp = c->st.Mp;
+  const int64_t ldc = c->chunk_cols, plane = (int64_t)Mp * ldc, MM = (int64_t)Mp * Mp;
+  ProfScope ps(c, PC_TRSM_BWD);
+  switch (pl.s5) {
+    case ENG_TF32: {
+      t5::EpiF5 e5{c->Ab.p, ldc};
+      t5::Args g{Mp, t5::KM_FROM_N, 0, 0, t5::MnDesc()};
+      return launch_t5<false, false>(c, dim3(ncols / t5::TM, Mp / t5::TN, 1), reinterpret_cast<float*>(c->fAb.p), plane, Mp, ncols,
+                                     reinterpret_cast<float*>(c->fLi.p), MM, Mp, Mp, g, e5);
+    }
+    case ENG_I8: {
+      // an exact-accumulation INT8 product with the explicit inverse: Ab (FP64, inducing-major, from the S4 epilogue) is cut into
+      // S5_NS slice planes per point, the product overwrites Ab with Kb
+      i8e::transpose_slice_kernel<i8e::S5_NS><<<(ncols + 31) / 32, 256, 0, c->stream>>>(c->Ab.p, ldc, Mp, ncols, reinterpret_cast<signed char*>(c->qAb.p), Mp,
+                                                                                      plane, c->sAb.p, c->sAb.p + ldc);
+      LAUNCHED(c);
+      KCHECK();
+      i8e::EpiE5 e5{c->Ab.p, ldc, c->sAb.p, c->sLi.p};
+      return launch_i8<i8e::EpiE5, i8e::S5_NS, i8e::S5_N>(c, c->qAb, ncols, plane, c->qLi, Mp, MM, Mp, dim3(Mp / i8e::S5_N, ncols / i8e::EM, 1),
+                                                          i8e::Args{Mp, i8e::KM_FROM_N, 0, 0}, e5);
+    }
+    default:
+      return solve_lk<TR_RHS_BWD>(c, c->Ab.p, ldc, ncols / BN);
+  }
+}
+
+// S6: G += As A^T, one partial G per split of the points.  After a TF32 S4, whose epilogue leaves it out, g += A dmu follows.
+static int32_t sweep_s6(agp_ctx* c, const SweepPlan& pl, int ncols) {
+  const int Mp = c->st.Mp, nb = c->st.nb;
+  const int64_t ldc = c->chunk_cols, plane = (int64_t)Mp * ldc;
+  float* fA = reinterpret_cast<float*>(c->fA.p);
+  {
+    ProfScope ps(c, PC_SYRK);
+    switch (pl.s6) {
+      case ENG_TF32: {
+        const int kchunk = (int)round_up((ncols + c->nsplit - 1) / c->nsplit, t5::TM);
+        const int nz = (ncols + kchunk - 1) / kchunk;
+        t5::EpiF6 e6{c->Gpart.p, Mp};
+        t5::Args g{ncols, t5::KM_SPLIT, kchunk, 1, t5::MnDesc()};
+        OK((launch_t5<true, true>(c, dim3(Mp / t5::TM, Mp / t5::TN, nz), reinterpret_cast<float*>(c->fAs.p), plane, Mp, ncols, fA, plane, Mp, ncols, g, e6)));
+        break;
+      }
+      case ENG_I8: {
+        // Operands are already K-major (points contiguous): row maxima -> power-of-two scales -> seven 7-bit slice planes each for As
+        // (A operand, 128-row tiles) and A (B operand, 64-row tiles); one slab of 16384 points per blockIdx.z (INT32 accumulators:
+        // 7 * 127^2 * 16384 < 2^31), partial G per slab, summed in a fixed order with the other slabs
+        const int64_t ldk = round_up(ncols, 128), pbytes = (int64_t)Mp * ldk;
+        OK(c->q6A.ensure(((int64_t)i8e::S * pbytes + 7) / 8));
+        OK(c->q6As.ensure(((int64_t)i8e::S * pbytes + 7) / 8));
+        OK(c->s6.ensure(4 * (int64_t)Mp));
+        double* sA = c->s6.p;
+        double* sAs = c->s6.p + Mp;
+        unsigned long long* mx = reinterpret_cast<unsigned long long*>(c->s6.p + 2 * Mp);
+        CU(cudaMemsetAsync(mx, 0, sizeof(unsigned long long) * 2 * Mp, c->stream));
+        const int seg = 8192;
+        const dim3 gmx((ncols + seg - 1) / seg, Mp / 8);
+        i8e::rowmax_kernel<<<gmx, 256, 0, c->stream>>>(c->A.p, ldc, Mp, ncols, seg, mx);
+        LAUNCHED(c);
+        i8e::rowmax_kernel<<<gmx, 256, 0, c->stream>>>(c->As.p, ldc, Mp, ncols, seg, mx + Mp);
+        LAUNCHED(c);
+        const dim3 gsl((unsigned)((ldk + 1023) / 1024), Mp);
+        i8e::slice_rows2d_kernel<i8e::S><<<gsl, 256, 0, c->stream>>>(c->A.p, ldc, ncols, reinterpret_cast<signed char*>(c->q6A.p), ldk, pbytes, mx, sA);
+        LAUNCHED(c);
+        i8e::slice_rows2d_kernel<i8e::S><<<gsl, 256, 0, c->stream>>>(c->As.p, ldc, ncols, reinterpret_cast<signed char*>(c->q6As.p), ldk, pbytes, mx + Mp, sAs);
+        LAUNCHED(c);
+        KCHECK();
+        const int kchunk = 16384, nz = (int)((ldk + kchunk - 1) / kchunk);
+        if (nz > c->nsplit) return fail(AGP_ERR_ALLOC, "S6 (INT8): %d slabs of G needed, %d allocated", nz, c->nsplit);
+        i8e::EpiE6 e6{c->Gpart.p, Mp, sAs, sA};
+        OK((launch_i8<i8e::EpiE6>(c, c->q6As, Mp, pbytes, c->q6A, Mp, pbytes, ldk, dim3(Mp / i8e::EN, Mp / i8e::EM, nz),
+                                  i8e::Args{(int)ldk, i8e::KM_SPLIT, kchunk, 1}, e6)));
+        break;
+      }
+      default: {
+        SyrkArgs s{};
+        s.As = c->As.p;
+        s.A = c->A.p;
+        s.ld = ldc;
+        s.ncols = ncols;
+        s.kchunk = (int)round_up((ncols + c->nsplit - 1) / c->nsplit, BK);
+        s.G = c->Gpart.p;
+        s.Mp = Mp;
+        using Cfg = StageCfg<A_MK, B_NK>;
+        OK((ensure_smem<syrk_kernel>(c, Cfg::smem_bytes)));
+        syrk_kernel<<<dim3(nb * (nb + 1), c->nsplit), NTHREADS, Cfg::smem_bytes, c->stream>>>(s);
+        LAUNCHED(c);
+        KCHECK();
+      }
+    }
+  }
+  if (pl.s4 == ENG_TF32) {
+    ProfScope ps(c, PC_F32_AUX);
+    const int slab = 512, nslab = (ncols + slab - 1) / slab;
+    t5::gvec_kernel<<<dim3((Mp / 4 + 255) / 256, nslab), 256, 0, c->stream>>>(fA, fA + plane, Mp, Mp, c->dmu.p, ncols, slab, c->gpart.p, Mp);
+    LAUNCHED(c);
+    KCHECK();
+  }
+  return AGP_OK;
+}
+
+// S7: contraction of Kb with the kernel derivatives
+static int32_t sweep_s7(agp_ctx* c, const SweepPlan& pl, const double* pts, int npts) {
+  const bool dk = pl.s7_streamed && c->st.kp.kind != AGP_KERNEL_SE;
+  ProfScope ps(c, PC_KGRAD);
+  return run_kgrad(c, c->Ab.p, c->chunk_cols, pts, npts, (npts + 2047) / 2048, pl.s7_streamed ? c->Kf.p : nullptr, dk ? c->DKb.p : nullptr);
+}
+
+// local reductions of the reverse pass's partial sums into the packed reduce buffer
+static int32_t sweep_reduce(agp_ctx* c, const RedLayout& rl) {
+  const int Mp = c->st.Mp;
+  const int64_t MM = (int64_t)Mp * Mp;
+  sum_slices_kernel<<<(Mp + 255) / 256, 256, 0, c->stream>>>(c->gpart.p, (int)(c->chunk_cols / BN), Mp, Mp, c->red.p + rl.g);
+  LAUNCHED(c);
+  KCHECK();
+  sum_slices_kernel<<<1024, 256, 0, c->stream>>>(c->Gpart.p, c->nsplit, MM, MM, c->red.p + rl.G);
+  LAUNCHED(c);
+  KCHECK();
+  return finish_kgrad(c, c->nslab, 1.0, c->red.p + rl.dZ, c->red.p + rl.theta);
+}
+
 // forward (+ backward) sweep over points [offset, offset+count) of ds.  predict != 0: only S1-S3 writing mu/var.
 static int32_t sweep_points(agp_ctx* c, const double* X, const double* y, int64_t count, bool grad, bool predict, double* mu_out,
                             double* var_out) {
-  SvgpState& st = c->st;
-  const int Mp = st.Mp, D = st.D, nb = st.nb;
+  const SweepPlan& pl = c->st.plan;
+  const int Mp = c->st.Mp, D = c->st.D;
   const int64_t MM = (int64_t)Mp * Mp;
   const int64_t cols = pick_chunk_cols(c, count);
   OK(ensure_sweep_workspace(c, cols, grad));
@@ -1481,8 +1805,7 @@ static int32_t sweep_points(agp_ctx* c, const double* X, const double* y, int64_
       OK(fill(c, c->kpart.p, (int64_t)c->nslab * Mp * kgrad_stride(D), 0.0));
     }
   }
-  const bool emu_s2 = st.f64_emu && !st.f32 && Mp >= 768;
-  if (emu_s2) {  // slices of the rows of Bt^T (columns of Bt, contiguous in the column-major copy), one scale per column
+  if (pl.s2 == ENG_I8) {  // slices of the rows of Bt^T (columns of Bt, contiguous in the column-major copy), one scale per column
     OK(c->qBt7.ensure(((int64_t)i8e::S * MM + 7) / 8));
     OK(c->sBt7.ensure(Mp));
     i8e::slice_rows_kernel<i8e::S><<<(Mp + 7) / 8, 256, 0, c->stream>>>(c->Bt_cm.p, Mp, Mp, Mp, reinterpret_cast<signed char*>(c->qBt7.p), Mp, MM, c->sBt7.p);
@@ -1491,291 +1814,19 @@ static int32_t sweep_points(agp_ctx* c, const double* X, const double* y, int64_
   }
   for (int64_t lo = 0; lo < count; lo += cols) {
     const int npts = (int)std::min<int64_t>(cols, count - lo);
-    const int ncols = (int)round_up(npts, (st.f32 || st.f64_emu) ? 2 * BN : BN);  // Float32 mode: the tcgen05 stages tile the points by 128
-    const int tiles_n = ncols / BN;
-    const double* pts = X + lo * D;
-    // S1: A = Lk^-1 Kuf
-    TrsmArgs t1{};
-    t1.T = c->Lt.p;
-    t1.ldt = Mp;
-    t1.nb = nb;
-    t1.X = c->A.p;
-    t1.ldx = ldc;
-    t1.pts = pts;
-    t1.npts = npts;
-    t1.zsp = c->zsp.p;
-    t1.mt = c->mt.p;
-    t1.saa = c->saa.p;
-    t1.sam = c->sam.p;
-    t1.kp = st.kp;
-    const bool s1_i8 = st.f32 && !s1_fused() && Mp >= 768;
-    if (s1_i8) {  // (below M ~ 768 the DMMA solve is as fast: C2, M = 512: 11.5 against 12.0 ms)
-      // Float32 mode: A = Linv Kuf as an FP64-accurate INT8-slice product (i8emu.cuh, 7 slices): generator -> Kf (FP64, also S7's input),
-      // point-major slices with exact per-point scales, 28 exact slice products, column sums in the epilogue
-      ProfScope ps(c, PC_TRSM_FWD);
-      if (st.kp.kind != AGP_KERNEL_SE) OK(c->DKb.ensure((int64_t)Mp * ldc));  // (the generator also stores kappa' for the Matern kinds)
-      OK(launch_s1(c, t1, tiles_n, true, true));
-      signed char* qK = reinterpret_cast<signed char*>(c->qK.p);
-      const int64_t pbytes = (int64_t)Mp * ldc, MM8 = (int64_t)Mp * Mp;
-      i8e::transpose_slice_kernel<i8e::S><<<(ncols + 31) / 32, 256, 0, c->stream>>>(c->Kf.p, ldc, Mp, ncols, qK, Mp, pbytes, c->sK.p);
-      LAUNCHED(c);
-      KCHECK();
-      CUtensorMap ma, mb;
-      if (!i8e::make_map3(&ma, qK, Mp, ncols, Mp, pbytes, i8e::EM, i8e::S) ||
-          !i8e::make_map3(&mb, reinterpret_cast<signed char*>(c->qLi7.p), Mp, Mp, Mp, MM8, i8e::EN, i8e::S))
-        return fail(AGP_ERR_CUDA, "cuTensorMapEncodeTiled failed");
-      const int nparts = Mp / 32;
-      i8e::EpiE1 e1{c->A.p, ldc, c->sK.p, c->sLi7.p, c->mt.p, c->sxx_part.p, c->sxx_part.p + (int64_t)nparts * ldc, ldc};
-      // the TF32 planes of A come straight from this epilogue
-      e1.Ah = reinterpret_cast<float*>(c->fA.p);
-      e1.Al = e1.Ah + (int64_t)Mp * ldc;
-      e1.ldf = Mp;
-      i8e::Args g8{Mp, i8e::KM_UPTO_N, 0, 0};
-      OK((ensure_smem<i8e::i8emu_gemm_kernel<i8e::EpiE1>>(c, i8e::SMEM_BYTES)));
-      i8e::i8emu_gemm_kernel<i8e::EpiE1><<<dim3(Mp / i8e::EN, ncols / i8e::EM, 1), i8e::E_THREADS, i8e::SMEM_BYTES, c->stream>>>(ma, mb, g8, e1);
-      LAUNCHED(c);
-      KCHECK();
-      i8e::colsum_reduce_kernel<<<(ncols + 255) / 256, 256, 0, c->stream>>>(c->sxx_part.p, nparts, ldc, ncols, c->saa.p, c->sam.p);
-      LAUNCHED(c);
-      KCHECK();
-    } else {
-      ProfScope ps(c, PC_TRSM_FWD);
-      OK(launch_s1(c, t1, tiles_n, grad && kgrad_fast(st)));
-    }
-    // Float32 mode: point-major hi / lo planes of A, then C = A Bt on the tcgen05 path (f32sweep.cuh)
-    const int64_t plane = (int64_t)Mp * ldc;  // floats per plane
-    float* fA = reinterpret_cast<float*>(c->fA.p);
-    float* fC = reinterpret_cast<float*>(c->fC.p);
-    float* fAb = reinterpret_cast<float*>(c->fAb.p);
-    float* fAs = reinterpret_cast<float*>(c->fAs.p);
-    const int64_t MMf = (int64_t)Mp * Mp;
-    const dim3 grid5(ncols / t5::TM, Mp / t5::TN, 1);
-    if (st.f32) {
-      if (!s1_i8) {
-        ProfScope ps(c, PC_F32_AUX);
-        t5::transpose_split_kernel<<<dim3(ncols / 32, Mp / 32), 256, 0, c->stream>>>(c->A.p, ldc, Mp, ncols, fA, fA + plane, Mp);
-        LAUNCHED(c);
-        KCHECK();
-      }
-      ProfScope ps(c, PC_GEMM_BTA);
-      t5::EpiF2 e2{fC, fC + plane, Mp, c->scc_part.p, ldc};
-      t5::Args g{Mp, t5::KM_FROM_N, 0, 0, t5::MnDesc()};
-      OK((launch_t5<false, false>(c, grid5, fA, plane, Mp, ncols, reinterpret_cast<float*>(c->fBtc.p), MMf, Mp, Mp, g, e2)));
-    } else if (emu_s2 && ncols >= 2048) {
-      // AGP_COMPUTE_F64_EMU, S2: C[n][j] = sum_{l >= j} A[n][l] Bt[l][j] on the INT8 engine.  The point-major slice planes of A live in the
-      // buffer that S6 refills with its own planes later in this launch group.
-      ProfScope ps(c, PC_GEMM_BTA);
-      const int64_t pbytes = (int64_t)Mp * ldc;
-      OK(c->q6As.ensure(((int64_t)i8e::S * pbytes + 7) / 8));
-      OK(c->sPm.ensure(ldc));
-      signed char* qApm = reinterpret_cast<signed char*>(c->q6As.p);
-      i8e::transpose_slice_kernel<i8e::S><<<(ncols + 31) / 32, 256, 0, c->stream>>>(c->A.p, ldc, Mp, ncols, qApm, Mp, pbytes, c->sPm.p);
-      LAUNCHED(c);
-      KCHECK();
-      CUtensorMap ma, mb;
-      if (!i8e::make_map3(&ma, qApm, Mp, ncols, Mp, pbytes, i8e::EM, i8e::S) ||
-          !i8e::make_map3(&mb, reinterpret_cast<signed char*>(c->qBt7.p), Mp, Mp, Mp, MM, i8e::EN, i8e::S))
-        return fail(AGP_ERR_CUDA, "cuTensorMapEncodeTiled failed");
-      i8e::EpiE2 e2{c->C.p, ldc, c->sPm.p, c->sBt7.p, c->scc_part.p, ldc};
-      i8e::Args g8{Mp, i8e::KM_FROM_N, 0, 0};
-      OK((ensure_smem<i8e::i8emu_gemm_kernel<i8e::EpiE2>>(c, i8e::SMEM_BYTES)));
-      i8e::i8emu_gemm_kernel<i8e::EpiE2><<<dim3(Mp / i8e::EN, ncols / i8e::EM, 1), i8e::E_THREADS, i8e::SMEM_BYTES, c->stream>>>(ma, mb, g8, e2);
-      LAUNCHED(c);
-      KCHECK();
-    } else {
-    // S2: C = Bt^T A  (A operand (m=j, k=l) = Bt[l][j] = Bt_rm[l*Mp + j]; nonzero for l >= j)
-    EpiS2 e2{c->C.p, ldc, c->scc_part.p, ldc};
-    {
-      ProfScope ps(c, PC_GEMM_BTA);
-      OK((run_gemm<A_KM, B_KN>(c, nb, tiles_n, c->Bt_rm.p, Mp, c->A.p, ldc, Mp, KR_UPPER, TS_ALL, e2)));
-    }
-    }
-    // S3: per-point stage
-    PerPointArgs pp{};
-    pp.saa = c->saa.p;
-    pp.sam = c->sam.p;
-    pp.scc_part = c->scc_part.p;
-    pp.ldp = ldc;
-    pp.nb = st.f32 ? 2 * nb : ((emu_s2 && ncols >= 2048) ? 4 * nb : nb);
-    pp.pts = pts;
-    pp.y = y ? y + lo : nullptr;
-    pp.npts = npts;
-    pp.ncols = ncols;
-    pp.scale = st.scale;
-    pp.mean_const = st.mean_const;
-    pp.kp = st.kp;
-    pp.lp = st.lp;
-    pp.dmu = c->dmu.p;
-    pp.dv = c->dv.p;
-    pp.mu_out = mu_out ? mu_out + lo : nullptr;
-    pp.var_out = var_out ? var_out + lo : nullptr;
-    pp.sc_part = c->sc_part.p;
-    pp.flag = c->d_flags + 1;
-    pp.predict_only = predict ? 1 : 0;
-    pp.point0 = c->st.point_base + lo;
-    const int pblocks = (ncols + PP_POINTS_PER_BLOCK - 1) / PP_POINTS_PER_BLOCK;
-    {
-      ProfScope ps(c, PC_PERPOINT);
-      perpoint_kernel<<<pblocks, 256, 0, c->stream>>>(pp);
-      LAUNCHED(c);
-      KCHECK();
-      if (predict) continue;
-      const int nsc_used = st.kp.kind == AGP_KERNEL_LINEAR ? SC_DS + D : SC_DS;
-      scal_reduce_kernel<<<1, 256, 0, c->stream>>>(c->sc_part.p, pblocks, nsc_used, c->red.p + rl.scal);
-      LAUNCHED(c);
-      KCHECK();
-    }
-    if (!grad) continue;
-    if (st.f32) {
-      const bool s5t = st.f32_tc_solve;
-      {
-        ProfScope ps(c, PC_GEMM_BC);
-        t5::Args g{Mp, t5::KM_UPTO_N, 0, 0, t5::MnDesc()};
-        if (s5t) {
-          t5::EpiF4<true> e4{fA, fA + plane, fAb, fAb + plane, fAs, fAs + plane, Mp, c->dmu.p, c->dv.p, c->mt.p, c->Ab.p, ldc};
-          OK((launch_t5<false, false>(c, grid5, fC, plane, Mp, ncols, reinterpret_cast<float*>(c->fBtr.p), MMf, Mp, Mp, g, e4)));
-        } else {
-          t5::EpiF4<false> e4{fA, fA + plane, fAb, fAb + plane, fAs, fAs + plane, Mp, c->dmu.p, c->dv.p, c->mt.p, c->Ab.p, ldc};
-          // the column maxima of Ab ride along: the INT8 S5 slices without a pass of its own for them
-          CU(cudaMemsetAsync(c->sAb.p + ldc, 0, sizeof(double) * ncols, c->stream));
-          e4.abmax = c->sAb.p + ldc;
-          OK((launch_t5<false, false>(c, grid5, fC, plane, Mp, ncols, reinterpret_cast<float*>(c->fBtr.p), MMf, Mp, Mp, g, e4)));
-        }
-      }
-      if (s5t) {
-        ProfScope ps(c, PC_TRSM_BWD);
-        t5::EpiF5 e5{c->Ab.p, ldc};
-        t5::Args g{Mp, t5::KM_FROM_N, 0, 0, t5::MnDesc()};
-        OK((launch_t5<false, false>(c, grid5, fAb, plane, Mp, ncols, reinterpret_cast<float*>(c->fLi.p), MMf, Mp, Mp, g, e5)));
-      } else {
-        // Kb = Lk^-T Ab as an exact-accumulation INT8 product with the explicit inverse: Ab (FP64, inducing-major, from the S4 epilogue) is
-        // cut into 4 slice planes per point (transpose_slice_kernel), the product overwrites Ab with Kb
-        ProfScope ps(c, PC_TRSM_BWD);
-        signed char* qAb = reinterpret_cast<signed char*>(c->qAb.p);
-        const int64_t pbytes = (int64_t)Mp * ldc;
-        i8e::transpose_slice_kernel<i8e::S5_NS><<<(ncols + 31) / 32, 256, 0, c->stream>>>(c->Ab.p, ldc, Mp, ncols, qAb, Mp, pbytes, c->sAb.p, c->sAb.p + ldc);
-        LAUNCHED(c);
-        KCHECK();
-        CUtensorMap ma, mb;
-        if (!i8e::make_map3(&ma, qAb, Mp, ncols, Mp, pbytes, i8e::EM, i8e::S5_NS) ||
-            !i8e::make_map3(&mb, reinterpret_cast<signed char*>(c->qLi.p), Mp, Mp, Mp, MM, i8e::S5_N, i8e::S5_NS))
-          return fail(AGP_ERR_CUDA, "cuTensorMapEncodeTiled failed");
-        i8e::EpiE5 e5{c->Ab.p, ldc, c->sAb.p, c->sLi.p};
-        i8e::Args g8{Mp, i8e::KM_FROM_N, 0, 0};
-        constexpr int sm8 = i8e::Cfg<i8e::S5_NS, i8e::S5_N>::smem_bytes;
-        OK((ensure_smem<i8e::i8emu_gemm_kernel<i8e::EpiE5, i8e::S5_NS, i8e::S5_N>>(c, sm8)));
-        i8e::i8emu_gemm_kernel<i8e::EpiE5, i8e::S5_NS, i8e::S5_N><<<dim3(Mp / i8e::S5_N, ncols / i8e::EM, 1), i8e::E_THREADS, sm8, c->stream>>>(ma, mb, g8, e5);
-        LAUNCHED(c);
-        KCHECK();
-      }
-      {
-        ProfScope ps(c, PC_SYRK);
-        const int kchunk = (int)round_up((ncols + c->nsplit - 1) / c->nsplit, t5::TM);
-        const int nz = (ncols + kchunk - 1) / kchunk;
-        t5::EpiF6 e6{c->Gpart.p, Mp};
-        t5::Args g{ncols, t5::KM_SPLIT, kchunk, 1, t5::MnDesc()};
-        OK((launch_t5<true, true>(c, dim3(Mp / t5::TM, Mp / t5::TN, nz), fAs, plane, Mp, ncols, fA, plane, Mp, ncols, g, e6)));
-      }
-      {
-        ProfScope ps(c, PC_F32_AUX);
-        const int slab = 512, nslab = (ncols + slab - 1) / slab;
-        t5::gvec_kernel<<<dim3((Mp / 4 + 255) / 256, nslab), 256, 0, c->stream>>>(fA, fA + plane, Mp, Mp, c->dmu.p, ncols, slab, c->gpart.p, Mp);
-        LAUNCHED(c);
-        KCHECK();
-      }
-    } else {
-    // S4: Ab = dmu (x) mt + 2 dv (Bt C - A), As = dv A, g partial   (A operand (m=j,k=l) = Bt[j][l], l <= j)
-    EpiS4 e4{c->A.p, c->Ab.p, c->As.p, ldc, c->dmu.p, c->dv.p, c->mt.p, c->gpart.p, Mp};
-    {
-      ProfScope ps(c, PC_GEMM_BC);
-      OK((run_gemm<A_KM, B_KN>(c, nb, tiles_n, c->Bt_cm.p, Mp, c->C.p, ldc, Mp, KR_LOWER, TS_ALL, e4)));
-    }
-    // S5: Kb = Lk^-T Ab (in place)
-    TrsmArgs t5a{};
-    t5a.T = c->Ut.p;
-    t5a.ldt = Mp;
-    t5a.nb = nb;
-    t5a.X = c->Ab.p;
-    t5a.ldx = ldc;
-    t5a.kp = st.kp;
-    {
-      ProfScope ps(c, PC_TRSM_BWD);
-      OK(launch_trsm<TR_RHS_BWD>(c, t5a, tiles_n));
-    }
-    // S6: G += As A^T
-    if (st.f64_emu && Mp >= 768 && ncols >= 2048) {  // (at M = 512 the DMMA SYRK is as fast: C2 10.7 against 11.3 ms; C4 350 -> 250 ms, C5 minibatch 139 -> 74 ms)
-      // AGP_COMPUTE_F64_EMU: the FP64-accurate INT8 engine (i8emu.cuh) over the points of the launch group.  Operands are already K-major (points contiguous):
-      // row maxima -> power-of-two scales -> seven 7-bit slice planes each for As (A operand, 128-row tiles) and A (B operand, 64-row tiles); one slab of
-      // 16384 points per blockIdx.z (INT32 accumulators: 7 * 127^2 * 16384 < 2^31), partial G per slab, summed in a fixed order with the other slabs
-      ProfScope ps(c, PC_SYRK);
-      const int64_t ldk = round_up(ncols, 128), pbytes = (int64_t)Mp * ldk;
-      OK(c->q6A.ensure(((int64_t)i8e::S * pbytes + 7) / 8));
-      OK(c->q6As.ensure(((int64_t)i8e::S * pbytes + 7) / 8));
-      OK(c->s6.ensure(4 * (int64_t)Mp));
-      double* sA = c->s6.p;
-      double* sAs = c->s6.p + Mp;
-      unsigned long long* mx = reinterpret_cast<unsigned long long*>(c->s6.p + 2 * Mp);
-      CU(cudaMemsetAsync(mx, 0, sizeof(unsigned long long) * 2 * Mp, c->stream));
-      const int seg = 8192;
-      const dim3 gmx((ncols + seg - 1) / seg, Mp / 8);
-      i8e::rowmax_kernel<<<gmx, 256, 0, c->stream>>>(c->A.p, ldc, Mp, ncols, seg, mx);
-      i8e::rowmax_kernel<<<gmx, 256, 0, c->stream>>>(c->As.p, ldc, Mp, ncols, seg, mx + Mp);
-      signed char* qA = reinterpret_cast<signed char*>(c->q6A.p);
-      signed char* qAs = reinterpret_cast<signed char*>(c->q6As.p);
-      const dim3 gsl((unsigned)((ldk + 1023) / 1024), Mp);
-      i8e::slice_rows2d_kernel<i8e::S><<<gsl, 256, 0, c->stream>>>(c->A.p, ldc, ncols, qA, ldk, pbytes, mx, sA);
-      i8e::slice_rows2d_kernel<i8e::S><<<gsl, 256, 0, c->stream>>>(c->As.p, ldc, ncols, qAs, ldk, pbytes, mx + Mp, sAs);
-      c->launches += 4;
-      KCHECK();
-      CUtensorMap ma, mb;
-      if (!i8e::make_map3(&ma, qAs, ldk, Mp, ldk, pbytes, i8e::EM, i8e::S) || !i8e::make_map3(&mb, qA, ldk, Mp, ldk, pbytes, i8e::EN, i8e::S))
-        return fail(AGP_ERR_CUDA, "cuTensorMapEncodeTiled failed");
-      const int kchunk = 16384, nz = (int)((ldk + kchunk - 1) / kchunk);
-      if (nz > c->nsplit) return fail(AGP_ERR_ALLOC, "S6 (INT8): %d slabs of G needed, %d allocated", nz, c->nsplit);
-      i8e::EpiE6 e6{c->Gpart.p, Mp, sAs, sA};
-      i8e::Args g8{(int)ldk, i8e::KM_SPLIT, kchunk, 1};
-      OK((ensure_smem<i8e::i8emu_gemm_kernel<i8e::EpiE6>>(c, i8e::SMEM_BYTES)));
-      i8e::i8emu_gemm_kernel<i8e::EpiE6><<<dim3(Mp / i8e::EN, Mp / i8e::EM, nz), i8e::E_THREADS, i8e::SMEM_BYTES, c->stream>>>(ma, mb, g8, e6);
-      LAUNCHED(c);
-      KCHECK();
-    } else {
-      ProfScope ps(c, PC_SYRK);
-      SyrkArgs s{};
-      s.As = c->As.p;
-      s.A = c->A.p;
-      s.ld = ldc;
-      s.ncols = ncols;
-      s.kchunk = (int)round_up((ncols + c->nsplit - 1) / c->nsplit, BK);
-      s.G = c->Gpart.p;
-      s.Mp = Mp;
-      using Cfg = StageCfg<A_MK, B_NK>;
-      OK((ensure_smem<syrk_kernel>(c, Cfg::smem_bytes)));
-      dim3 grid(nb * (nb + 1), c->nsplit);
-      syrk_kernel<<<grid, NTHREADS, Cfg::smem_bytes, c->stream>>>(s);
-      LAUNCHED(c);
-      KCHECK();
-    }
-    }
-    // S7: contraction of Kb with the kernel derivatives
-    {
-      ProfScope ps(c, PC_KGRAD);
-      if (kgrad_fast(st)) {
-        OK(run_kgrad(c, c->Ab.p, ldc, pts, npts, (npts + 2047) / 2048, c->Kf.p, st.kp.kind != AGP_KERNEL_SE ? c->DKb.p : nullptr));
-      } else {
-        OK(run_kgrad(c, c->Ab.p, ldc, pts, npts, (npts + 2047) / 2048));
-      }
-    }
+    const int ncols = (int)round_up(npts, pl.pts_tile);
+    const SweepPlan gp = pl.at_width(ncols);
+    OK(sweep_s1(c, gp, X + lo * D, npts, ncols, grad && gp.s7_streamed));
+    OK(sweep_s2(c, gp, ncols));
+    OK(sweep_s3(c, gp, X, y, lo, npts, ncols, predict, mu_out, var_out, c->red.p + rl.scal));
+    if (predict || !grad) continue;
+    OK(sweep_s4(c, gp, ncols));
+    OK(sweep_s5(c, gp, ncols));
+    OK(sweep_s6(c, gp, ncols));
+    OK(sweep_s7(c, gp, X + lo * D, npts));
   }
   if (predict || !grad) return AGP_OK;
-  // local reductions into the packed buffer
-  sum_slices_kernel<<<(Mp + 255) / 256, 256, 0, c->stream>>>(c->gpart.p, (int)(ldc / BN), Mp, Mp, c->red.p + rl.g);
-  LAUNCHED(c);
-  KCHECK();
-  sum_slices_kernel<<<1024, 256, 0, c->stream>>>(c->Gpart.p, c->nsplit, MM, MM, c->red.p + rl.G);
-  LAUNCHED(c);
-  KCHECK();
-  OK(finish_kgrad(c, c->nslab, 1.0, c->red.p + rl.dZ, c->red.p + rl.theta));
-  return AGP_OK;
+  return sweep_reduce(c, rl);
 }
 
 static int32_t check_dataset(agp_ctx* c, agp_dataset* ds, int64_t offset, int64_t count, int D) {
@@ -1864,14 +1915,7 @@ extern "C" int32_t agp_svgp_finish(agp_ctx* c, double* elbo_out, agp_svgp_grads*
   OK((run_gemm<A_KM, B_KN>(c, nb, Mp / BN, W1, Mp, G, Mp, Mp, KR_FULL, TS_ALL,
                            epi_store(W2, Mp, true, 2.0, 0.0, MASK_NONE, 0.0, c->mt.p, g, 1.0))));
   // W2 <- V = Lk^-T Asum
-  TrsmArgs tb{};
-  tb.T = c->Ut.p;
-  tb.ldt = Mp;
-  tb.nb = nb;
-  tb.ldx = Mp;
-  tb.kp = st.kp;
-  tb.X = W2;
-  OK(launch_trsm<TR_RHS_BWD>(c, tb, Mp / BN));
+  OK(solve_lk<TR_RHS_BWD>(c, W2, Mp, Mp / BN));
   // W3 (row-major) = Bt-bar = tril(2 G Bt) [- Bt if centered]
   //   B operand (k, n) = Bt[k][n] = Bt_rm[k*Mp + n]
   OK((run_gemm<A_KM, B_KN>(c, nb, Mp / BN, G, Mp, c->Bt_rm.p, Mp, Mp, KR_FULL, TS_ALL, epi_store(W3, Mp, true, 2.0, 0.0, MASK_LOWER))));
@@ -1888,9 +1932,7 @@ extern "C" int32_t agp_svgp_finish(agp_ctx* c, double* elbo_out, agp_svgp_grads*
     vec_to_rhs_kernel<<<(Mp * 64 + 255) / 256, 256, 0, c->stream>>>(c->vec64b.p, 0.0, Mp, Mp, c->vec64.p);
     LAUNCHED(c);
     KCHECK();
-    tb.X = c->vec64.p;
-    tb.ldx = 64;
-    OK(launch_trsm<TR_RHS_BWD>(c, tb, 1));
+    OK(solve_lk<TR_RHS_BWD>(c, c->vec64.p, 64, 1));
     rhs_to_vec_kernel<<<(Mp + 255) / 256, 256, 0, c->stream>>>(c->vec64.p, Mp, c->vec64b.p + Mp);  // m-bar in vec64b[Mp..2Mp)
     LAUNCHED(c);
     KCHECK();
@@ -1898,9 +1940,7 @@ extern "C" int32_t agp_svgp_finish(agp_ctx* c, double* elbo_out, agp_svgp_grads*
     LAUNCHED(c);
     KCHECK();
     // W3 <- Y = Lk^-T Bt-bar (row-major, in place)
-    tb.X = W3;
-    tb.ldx = Mp;
-    OK(launch_trsm<TR_RHS_BWD>(c, tb, Mp / BN));
+    OK(solve_lk<TR_RHS_BWD>(c, W3, Mp, Mp / BN));
     // W4 (row-major) = X2 = Y Bt^T + m-bar mt^T ;  A operand (m,k) = Y[m][k] row-major (MK); B (k,n) = Bt[n][k] = Bt_cm[n + k*Mp]
     OK((run_gemm<A_MK, B_KN>(c, nb, Mp / BN, W3, Mp, c->Bt_cm.p, Mp, Mp, KR_FULL, TS_ALL,
                              epi_store(W4, Mp, true, 1.0, 0.0, MASK_NONE, 0.0, c->vec64b.p + Mp, c->mt.p, 1.0))));
@@ -1915,12 +1955,9 @@ extern "C" int32_t agp_svgp_finish(agp_ctx* c, double* elbo_out, agp_svgp_grads*
   // W2 (row-major) = Phi(Lk^T Lk-bar);  A operand (m,k) = Lk[k][m] = Lk_cm[k + m*Mp] (MK), nonzero for k >= m
   OK((run_gemm<A_MK, B_KN>(c, nb, Mp / BN, c->Lk.p, Mp, W1, Mp, Mp, KR_UPPER, TS_ALL, epi_store(W2, Mp, true, 1.0, 0.0, MASK_PHI))));
   // Y1 = Lk^-T W2 ; Y2 = Lk^-T Y1^T ; Kuu-bar = (Y2 + Y2^T)/2
-  tb.X = W2;
-  tb.ldx = Mp;
-  OK(launch_trsm<TR_RHS_BWD>(c, tb, Mp / BN));
+  OK(solve_lk<TR_RHS_BWD>(c, W2, Mp, Mp / BN));
   OK(transpose(c, W2, W1, Mp, Mp));
-  tb.X = W1;
-  OK(launch_trsm<TR_RHS_BWD>(c, tb, Mp / BN));
+  OK(solve_lk<TR_RHS_BWD>(c, W1, Mp, Mp / BN));
   OK(transpose(c, W1, W2, Mp, Mp));
   sym_average_kernel<<<1024, 256, 0, c->stream>>>(W1, W2, W4, MM);  // W4 = Kuu-bar (symmetric)
   LAUNCHED(c);
@@ -2109,14 +2146,7 @@ extern "C" int32_t agp_svgp_posterior(agp_ctx* c, const agp_svgp_params* p, doub
     vec_to_rhs_kernel<<<(Mp * 64 + 255) / 256, 256, 0, c->stream>>>(c->mt.p, 0.0, Mp, Mp, c->vec64.p);
     LAUNCHED(c);
     KCHECK();
-    TrsmArgs tb{};
-    tb.T = c->Ut.p;
-    tb.ldt = Mp;
-    tb.nb = st.nb;
-    tb.X = c->vec64.p;
-    tb.ldx = 64;
-    tb.kp = st.kp;
-    OK(launch_trsm<TR_RHS_BWD>(c, tb, 1));
+    OK(solve_lk<TR_RHS_BWD>(c, c->vec64.p, 64, 1));
     rhs_to_vec_kernel<<<(Mp + 255) / 256, 256, 0, c->stream>>>(c->vec64.p, Mp, c->vec64b.p);
     LAUNCHED(c);
     KCHECK();
@@ -2157,20 +2187,7 @@ extern "C" int32_t agp_svgp_mean_and_var(agp_ctx* c, const agp_svgp_params* p, c
 // A = Lk^-1 Kuf and C = Bt^T A for one set of points (single chunk), into the given scratch matrices.
 static int32_t project_points(agp_ctx* c, const double* X_dev, int n, int ncols, double* Abuf, double* Cbuf, int64_t ldc) {
   SvgpState& st = c->st;
-  TrsmArgs t1{};
-  t1.T = c->Lt.p;
-  t1.ldt = st.Mp;
-  t1.nb = st.nb;
-  t1.X = Abuf;
-  t1.ldx = ldc;
-  t1.pts = X_dev;
-  t1.npts = n;
-  t1.zsp = c->zsp.p;
-  t1.mt = c->mt.p;
-  t1.saa = c->saa.p;
-  t1.sam = c->sam.p;
-  t1.kp = st.kp;
-  OK(launch_s1(c, t1, ncols / BN));
+  OK(launch_s1(c, s1_args(c, Abuf, ldc, X_dev, n), ncols / BN));
   EpiS2 e2{Cbuf, ldc, c->scc_part.p, ldc};
   OK((run_gemm<A_KM, B_KN>(c, st.nb, ncols / BN, c->Bt_rm.p, st.Mp, Abuf, ldc, st.Mp, KR_UPPER, TS_ALL, e2)));
   return AGP_OK;
@@ -2208,26 +2225,8 @@ extern "C" int32_t agp_svgp_mean_and_cov(agp_ctx* c, const agp_svgp_params* p, c
   KCHECK();
   OK(project_points(c, c->px1.p, (int)n1, n1p, c->A.p, c->C.p, ldc));
   if (mu1_out) {
-    PerPointArgs pp{};
-    pp.saa = c->saa.p;
-    pp.sam = c->sam.p;
-    pp.scc_part = c->scc_part.p;
-    pp.ldp = ldc;
-    pp.nb = st.nb;
-    pp.pts = c->px1.p;
-    pp.npts = (int)n1;
-    pp.ncols = n1p;
-    pp.scale = 1.0;
-    pp.mean_const = st.mean_const;
-    pp.kp = st.kp;
-    pp.lp = st.lp;
-    pp.mu_out = c->mu_out.p;
-    pp.var_out = c->var_out.p;
-    pp.flag = c->d_flags + 1;
-    pp.predict_only = 1;
-    perpoint_kernel<<<(n1p + PP_POINTS_PER_BLOCK - 1) / PP_POINTS_PER_BLOCK, 256, 0, c->stream>>>(pp);
-    LAUNCHED(c);
-    KCHECK();
+    // the per-point stage of the sweep in prediction mode; project_points ran S2 on DMMA
+    OK(sweep_s3(c, SweepPlan{}, c->px1.p, nullptr, 0, (int)n1, n1p, true, c->mu_out.p, c->var_out.p, nullptr));
     CU(cudaMemcpyAsync(mu1_out, c->mu_out.p, sizeof(double) * n1, cudaMemcpyDeviceToHost, c->stream));
   }
   const double *A2 = c->A.p, *C2 = c->C.p;

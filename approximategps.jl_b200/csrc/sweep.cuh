@@ -1,7 +1,7 @@
 // sweep.cuh -- the data-parallel SVGP sweep kernels (per chunk of points).
 //
-//   S1  trsm_kernel<TR_KUF_FWD>   A  = Lk^-1 Kuf   blocked left-looking TRSM; Kuf tiles are generated
-//                                 straight into the B-operand stage of the DMMA pipeline (never in HBM)
+//   S1  kuf_gen_kernel            Kuf of the launch group, written into the solution matrix (row-major)
+//       + trsm_kernel<TR_RHS_FWD_SUMS>  A = Lk^-1 Kuf in place (blocked left-looking TRSM)  + column a^T a, a^T mt
 //   S2  gemm + EpiS2              C  = Bt^T A       (upper-triangular operand)        + column |c|^2
 //   S3  perpoint_kernel           mu, var, E[log p], dE/dmu, dE/dvar                  (HBM-bound)
 //   S4  gemm + EpiS4              Ab = dmu (x) mt + 2 dv (Bt C - A),  As = dv A,  g += A dmu
@@ -18,7 +18,7 @@
 
 namespace agp {
 
-constexpr int TR_KUF_FWD = 0, TR_RHS_FWD = 1, TR_RHS_BWD = 2, TR_KUF_FWD_SCALED = 3, TR_RHS_FWD_SUMS = 4;
+constexpr int TR_RHS_FWD = 1, TR_RHS_BWD = 2, TR_KUF_FWD_SCALED = 3, TR_RHS_FWD_SUMS = 4;
 // TR_RHS_FWD_SUMS: the forward solve of S1 on a right-hand side that kuf_gen_kernel wrote into X (in place), with S1's column
 // sums a^T a and a^T mt.  The Kuf tile then costs one extra HBM write + read (0.6 GB per 151 552-point launch group, ~0.1 ms at
 // the measured copy bandwidth) instead of a generator entangled with the DMMA pipeline (~0.95 ms per launch group, r01t / r2a).
@@ -33,7 +33,7 @@ struct TrsmArgs {
   double* X;  // [Mp][ldx] row-major: solution (and, in RHS modes, the right-hand side; in place)
   int64_t ldx;
   const double* RHS;  // RHS modes, optional: right-hand side in a separate matrix (same layout); X is then only written / re-read as solution
-  // TR_KUF_FWD only
+  // the Kuf generator (kuf_gen_kernel, TR_KUF_FWD_SCALED) and S1's column sums
   const double* pts;  // chunk's points, point-major [npts][D]
   int npts;
   const double* zsp;  // [Mp][Dp + 2] padded scaled inducing inputs with their squared norm at column Dp (prep_z_kernel)
@@ -77,7 +77,6 @@ struct StepIter {
 // with ceil(D/4) k-steps each, fed straight from the padded z slab (A fragments) and x rows (B fragments); the
 // ||x||^2 + ||z||^2 - 2 x.z combination, the clamp and kappa are applied to the accumulator fragment, which is stored
 // as double2.  (Padded rows: kfun.cuh kuf_dp.)
-template <bool SCALED>
 __device__ __forceinline__ void gen_kuf_tile(double* __restrict__ sB, const double* __restrict__ sZ, const double* __restrict__ xs, int row0,
                                              const KernelParams& kp, int warp, int lane, const double* rowscale, const double* dvec, double (&pkd)[2]) {
   const int g = lane >> 2, t = lane & 3;
@@ -114,25 +113,22 @@ __device__ __forceinline__ void gen_kuf_tile(double* __restrict__ sB, const doub
     const bool valid = row < kp.M;
     double v0 = valid ? kp.variance * kappa_kp(kp, u[h][0]) : 0.0;
     double v1 = valid ? kp.variance * kappa_kp(kp, u[h][1]) : 0.0;
-    if (SCALED) {
-      const double dv = dvec[row], rsc = rowscale[row];
-      pkd[0] = fma(v0, dv, pkd[0]);
-      pkd[1] = fma(v1, dv, pkd[1]);
-      v0 *= rsc;
-      v1 *= rsc;
-    }
+    const double dv = dvec[row], rsc = rowscale[row];
+    pkd[0] = fma(v0, dv, pkd[0]);
+    pkd[1] = fma(v1, dv, pkd[1]);
+    v0 *= rsc;
+    v1 *= rsc;
     *reinterpret_cast<double2*>(sB + (g + 8 * h) * BTile<B_KN>::ld + c0) = make_double2(v0, v1);
   }
 }
 
-// Blocked left-looking triangular solve on one 64-column tile per CTA.  MODE TR_KUF_FWD generates its right-hand
-// side (the Kuf tile) on the fly; S = pipeline depth (4, or 3 when the z slabs of a wide input would not fit).
+// Blocked left-looking triangular solve on one 64-column tile per CTA.  MODE TR_KUF_FWD_SCALED generates its right-hand
+// side (the scaled Kuf tile) on the fly; S = pipeline depth (4, or 3 when the z slabs of a wide input would not fit).
 template <int MODE, int S>
 __global__ void __launch_bounds__(NTHREADS, 2) trsm_kernel(TrsmArgs a) {
   extern __shared__ __align__(128) double smem[];
   using Cfg = StageCfg<A_KM, B_KN>;
-  constexpr bool SCALED = MODE == TR_KUF_FWD_SCALED;
-  constexpr bool FWD = MODE == TR_KUF_FWD || SCALED;          // generator modes: the Kuf tile is built inside the pipeline
+  constexpr bool FWD = MODE == TR_KUF_FWD_SCALED;             // generator mode: the Kuf tile is built inside the pipeline
   constexpr bool SUMS = FWD || MODE == TR_RHS_FWD_SUMS;       // S1's column sums
   ThreadMap tm;
   const int tid = threadIdx.x;
@@ -178,7 +174,7 @@ __global__ void __launch_bounds__(NTHREADS, 2) trsm_kernel(TrsmArgs a) {
     __syncthreads();  // raw (stage 0) may be overwritten from here on
   }
 
-  double pkd[2] = {0.0, 0.0};  // SCALED: partial k' * dvec of this thread's 2 columns
+  double pkd[2] = {0.0, 0.0};  // FWD: partial k' * dvec of this thread's 2 columns
   StepIter it_issue, it_cons, it_gen;
   it_issue.init(MODE != TR_RHS_BWD, a.nb);
   it_cons.init(MODE != TR_RHS_BWD, a.nb);
@@ -205,7 +201,7 @@ __global__ void __launch_bounds__(NTHREADS, 2) trsm_kernel(TrsmArgs a) {
   };
   auto gen = [&](int slot) {  // it_gen describes the stage living in `slot`
     double* st = smem + slot * stage_elems;
-    gen_kuf_tile<SCALED>(st + Cfg::a_elems, st + Cfg::elems, xs, it_gen.J * BM + it_gen.kk * BK, a.kp, tm.warp, tm.lane, a.rowscale, a.dvec, pkd);
+    gen_kuf_tile(st + Cfg::a_elems, st + Cfg::elems, xs, it_gen.J * BM + it_gen.kk * BK, a.kp, tm.warp, tm.lane, a.rowscale, a.dvec, pkd);
   };
 
   Acc acc;
@@ -304,7 +300,7 @@ __global__ void __launch_bounds__(NTHREADS, 2) trsm_kernel(TrsmArgs a) {
       a.saa[n0 + tid] = ((sred[tid] + sred[64 + tid]) + sred[128 + tid]) + sred[192 + tid];
       a.sam[n0 + tid] = ((sred[256 + tid] + sred[320 + tid]) + sred[384 + tid]) + sred[448 + tid];
     }
-    if (SCALED) {
+    if (FWD) {
       // a thread holds the partial sums of columns 8 warp + 2 t + {0, 1} over its rows: reduce over g; no other warp
       // touches these columns
 #pragma unroll

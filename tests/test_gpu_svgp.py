@@ -501,41 +501,6 @@ def test_kernel_function_values(agp, kind):
             assert np.all(np.diag(got) == 1.3)  # exactly zero distances on the diagonal
 
 
-def test_fused_kuf_generator_variant_matches(agp):
-    """north_star's Kuf-never-in-HBM kernel (trsm_kernel<TR_KUF_FWD>: the tile generated inside the DMMA pipeline, X staged by a TMA bulk copy) is kept
-    behind AGP_S1_FUSED=1 (DESIGN.md section 2 explains why the stand-alone generator is the default: it is faster).  The knob is read once per process,
-    so the fused variant runs in a child process; both variants must agree with the oracle and with each other."""
-    import json
-    import subprocess
-
-    code = r'''
-import json, sys, os
-sys.path.insert(0, os.path.join(os.getcwd(), "tests")); sys.path.insert(0, os.getcwd())
-import numpy as np
-import agp_b200 as agp
-from _cases import agp_objects, make_problem
-out = {}
-for kind, D, M in (("se", 8, 300), ("matern52", 3, 140), ("linear", 2, 40)):
-    p = make_problem(seed=77, kind=kind, N=2000, M=M, D=D, lik="poisson_exp" if kind != "linear" else "gaussian", lengthscale=1.0 if D > 2 else None)
-    sva, lfx, quad, _ = agp_objects(agp, p)
-    v, g = agp.elbo_and_gradient(sva, lfx, p["y"], num_data=20000.0, quadrature=quad)
-    out[kind] = dict(elbo=v, m=g.m.tolist(), Z=g.Z.ravel().tolist(), variance=g.variance, ils=np.atleast_1d(g.inv_lengthscale).tolist())
-print("RESULT" + json.dumps(out))
-'''
-    res = {}
-    for fused in ("0", "1"):
-        env = dict(os.environ, AGP_S1_FUSED=fused)
-        r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, env=env, cwd=os.path.dirname(os.path.dirname(os.path.abspath(__file__))), timeout=600)
-        assert r.returncode == 0, r.stderr[-2000:]
-        res[fused] = json.loads([line for line in r.stdout.splitlines() if line.startswith("RESULT")][-1][6:])
-    for kind in res["0"]:
-        a, b = res["0"][kind], res["1"][kind]
-        assert abs(a["elbo"] - b["elbo"]) <= 1e-11 * abs(a["elbo"]), (kind, a["elbo"], b["elbo"])
-        for key in ("m", "Z", "ils"):
-            assert rel_err(np.array(b[key]), np.array(a[key])) < 1e-10, (kind, key)
-        assert abs(a["variance"] - b["variance"]) <= 1e-10 * max(1.0, abs(a["variance"]))
-
-
 @pytest.mark.parametrize("D,kind", [(12, "se"), (20, "matern52"), (32, "se"), (20, "linear")])
 def test_wide_inputs(agp, D, kind):
     """Input dimensions beyond 8 take the DMAX = 16 / 32 instantiations of the Kuf generator and of the streaming kernel-gradient kernel
