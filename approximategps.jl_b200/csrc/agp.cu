@@ -82,6 +82,16 @@ struct DevBuf {
   }
 };
 
+// n points padded with zero rows to np (a multiple of BM): raw x [np][D], scaled xs = s (.) x, squared norms xn and, for the Kuf generator,
+// the packed rows xsp (prep_z_kernel); filled by upload_points
+struct PointSet {
+  DevBuf x, xs, xn, xsp;
+  int n = 0, np = 0;
+  void release() {
+    for (DevBuf* b : {&x, &xs, &xn, &xsp}) b->release();
+  }
+};
+
 struct NcclApi {
   void* lib = nullptr;
   ncclResult_t (*GetUniqueId)(ncclUniqueId*) = nullptr;
@@ -140,7 +150,6 @@ struct SvgpState {
   bool sweep_pending = false;  // agp_svgp_sweep has filled the reduce buffer and agp_svgp_finish has not consumed it yet
   SweepPlan plan;
   int M = 0, Mp = 0, D = 0, nb = 0;
-  int n_scale = 1;
   bool centered = false;
   double mean_const = 0, jitter = 0, scale = 1;
   int want_grad = 0;
@@ -200,7 +209,8 @@ struct agp_ctx {
   int64_t chunk_cols = 0;  // capacity of the per-chunk scratch (columns)
   int nslab = 0, nsplit = 0;
   // once-per-step M x M operands (column-major, ld = Mp unless noted)
-  DevBuf z, zs, zn, zsp, mvec, mt, Lq, Kw, Lk, Lt, Ut, Bt_cm, Bt_rm, W1, W2, W3, W4, vec64, vec64b;
+  PointSet z;  // inducing points (SVGP) or training inputs (Laplace)
+  DevBuf mvec, mt, Lq, Kw, Lk, Lt, Ut, Bt_cm, Bt_rm, W1, W2, W3, W4, vec64, vec64b;
   // per-chunk scratch [Mp][chunk_cols]
   DevBuf A, C, Ab, As, saa, sam, scc_part, dmu, dv, sc_part;
   DevBuf Kf, DKb;  // reverse pass, stationary kernels: Kuf and variance * kappa'(u) of the launch group, kept from S1 for S7
@@ -217,7 +227,8 @@ struct agp_ctx {
   ncclComm_t comm = nullptr;
   int nranks = 1, rank = 0;
   // prediction outputs / scratch
-  DevBuf mu_out, var_out, px1, px2, pxs1, pxn1, pxs2, pxn2, pcov;
+  DevBuf mu_out, var_out, pcov;
+  PointSet px1, px2;
 };
 
 struct agp_dataset {
@@ -289,11 +300,12 @@ extern "C" int32_t agp_ctx_destroy(agp_ctx* c) {
   cudaSetDevice(c->device);
   cudaStreamSynchronize(c->stream);
   if (c->comm && g_nccl.CommDestroy) g_nccl.CommDestroy(c->comm);
-  DevBuf* bufs[] = {&c->z, &c->zs, &c->zn, &c->zsp, &c->mvec, &c->mt, &c->Lq, &c->Kw, &c->Lk, &c->Lt, &c->Ut, &c->Bt_cm, &c->Bt_rm,
+  DevBuf* bufs[] = {&c->mvec, &c->mt, &c->Lq, &c->Kw, &c->Lk, &c->Lt, &c->Ut, &c->Bt_cm, &c->Bt_rm,
                     &c->W1, &c->W2, &c->W3, &c->W4, &c->vec64, &c->vec64b, &c->A, &c->C, &c->Ab, &c->As, &c->Kf, &c->DKb, &c->saa, &c->sam,
                     &c->scc_part, &c->dmu, &c->dv, &c->sc_part, &c->gpart, &c->Gpart, &c->kpart, &c->red, &c->small, &c->ghbuf, &c->q6A, &c->q6As, &c->s6, &c->qBt7, &c->sBt7, &c->sPm, &c->fA, &c->fC, &c->fAb, &c->fAs, &c->fBtc, &c->fBtr, &c->fLi, &c->qAb, &c->sAb, &c->qLi, &c->sLi, &c->qK, &c->sK, &c->qLi7, &c->sLi7, &c->sxx_part,
-                    &c->mu_out, &c->var_out, &c->px1, &c->px2, &c->pxs1, &c->pxn1, &c->pxs2, &c->pxn2, &c->pcov};
+                    &c->mu_out, &c->var_out, &c->pcov};
   for (DevBuf* b : bufs) b->release();
+  for (PointSet* s : {&c->z, &c->px1, &c->px2}) s->release();
   lap_release(c);
   if (c->d_flags) cudaFree(c->d_flags);
   for (cudaEvent_t e : c->prof.pool) cudaEventDestroy(e);
@@ -676,6 +688,39 @@ static int32_t transpose(agp_ctx* c, const double* in, double* out, int n, int64
   return AGP_OK;
 }
 
+// n host points (point-major [n][kp.D]) -> ps, scaled by kp.s; packed: also the rows the Kuf generator streams
+static int32_t upload_points(agp_ctx* c, PointSet& ps, const double* host, int64_t n, KernelParams kp, bool packed) {
+  const int D = kp.D;
+  const int64_t np = round_up(n, BM);
+  OK(ps.x.ensure(np * D));
+  OK(ps.xs.ensure(np * D));
+  OK(ps.xn.ensure(np));
+  if (packed) OK(ps.xsp.ensure(np * (kuf_dp(D) + 2)));
+  CU(cudaMemsetAsync(ps.x.p, 0, sizeof(double) * np * D, c->stream));
+  CU(cudaMemcpyAsync(ps.x.p, host, sizeof(double) * n * D, cudaMemcpyHostToDevice, c->stream));
+  kp.M = (int)n;
+  prep_z_kernel<<<(int)((np + 127) / 128), 128, 0, c->stream>>>(ps.x.p, ps.xs.p, ps.xn.p, packed ? ps.xsp.p : nullptr, (int)np, kp);
+  LAUNCHED(c);
+  KCHECK();
+  ps.n = (int)n;
+  ps.np = (int)np;
+  return AGP_OK;
+}
+
+// cov(f.prior, a) + jitter I (the one-argument kernelmatrix: exactly zero distances on the diagonal; identity on the padding), or
+// cov(f.prior, a, b) (zero padding), into out: column-major, ld = a.np
+static int32_t prior_cov(agp_ctx* c, KernelParams kp, const PointSet& a, const PointSet* b, double jitter, double* out) {
+  if (b) {
+    cross_k_kernel<<<dim3((a.np + 127) / 128, b->np), 128, 0, c->stream>>>(out, a.np, a.xs.p, a.xn.p, a.n, b->xs.p, b->xn.p, b->n, a.np, kp);
+  } else {
+    kp.M = a.n;
+    build_kuu_kernel<<<dim3((a.np + 127) / 128, a.np), 128, 0, c->stream>>>(out, a.np, a.xs.p, a.xn.p, jitter, kp);
+  }
+  LAUNCHED(c);
+  KCHECK();
+  return AGP_OK;
+}
+
 // launch helpers use c->stream: point it at another stream for a scope
 struct StreamSwap {
   agp_ctx* c;
@@ -933,13 +978,41 @@ static int32_t blocked_cholesky(agp_ctx* c, double* Kw, double* L, double* Lt, d
   return AGP_OK;
 }
 
-// Lt off-diagonal blocks: Lt[J][L<J] = -inv(L_JJ) L[J][L];  Ut[J][L>J] = -(L[L][J] inv(L_JJ))^T
-static int32_t build_block_scaled(agp_ctx* c, const double* L, double* Lt, double* Ut, int nb, int64_t ld) {
+// Lt off-diagonal blocks: Lt[J][L<J] = -inv(L_JJ) L[J][L]
+static int32_t block_scale_lt(agp_ctx* c, const double* L, double* Lt, int nb, int64_t ld) {
   if (nb < 2) return AGP_OK;
   // A(m,k) = Lt diag block (column-major, KM); B(k,n) = L[(J*128+k) + n*ld]  (k contiguous: NK)
-  OK((run_gemm<A_KM, B_NK>(c, nb, 2 * nb, Lt, ld, L, ld, nb * BM, KR_DIAG, TS_NBLK_LT, epi_store(Lt, ld, false, -1.0))));
+  return run_gemm<A_KM, B_NK>(c, nb, 2 * nb, Lt, ld, L, ld, nb * BM, KR_DIAG, TS_NBLK_LT, epi_store(Lt, ld, false, -1.0));
+}
+// ... and Ut[J][L>J] = -(L[L][J] inv(L_JJ))^T
+static int32_t build_block_scaled(agp_ctx* c, const double* L, double* Lt, double* Ut, int nb, int64_t ld) {
+  if (nb < 2) return AGP_OK;
+  OK(block_scale_lt(c, L, Lt, nb, ld));
   // A(m,k) = Ut diag block = inv^T (KM); B(k,n) = L[n + (J*128+k)*ld]  (n contiguous: KN)
   OK((run_gemm<A_KM, B_KN>(c, nb, 2 * nb, Ut, ld, L, ld, nb * BM, KR_DIAG, TS_NBLK_GT, epi_store(Ut, ld, false, -1.0))));
+  return AGP_OK;
+}
+
+__global__ void set_diag_kernel(double* A, int n, int64_t ld, double v) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) A[(int64_t)i * ld + i] = v;
+}
+// Explicit inverse X = L^-1 (row-major [nb*BM]^2) of a blocked factor: the blocked TRSM against its block-scaled Lt on the identity.
+// Binv (optional, column-major) <- X^T X = (L L^T)^-1 by a triangular-aware GEMM.
+static int32_t factor_inverse(agp_ctx* c, const double* Lt, int nb, double* X, double* Binv = nullptr) {
+  const int np = nb * BM;
+  OK(fill(c, X, (int64_t)np * np, 0.0));
+  set_diag_kernel<<<(np + 255) / 256, 256, 0, c->stream>>>(X, np, np, 1.0);
+  LAUNCHED(c);
+  KCHECK();
+  TrsmArgs ta{};
+  ta.T = Lt;
+  ta.ldt = np;
+  ta.nb = nb;
+  ta.X = X;
+  ta.ldx = np;
+  OK(launch_trsm<TR_RHS_FWD>(c, ta, np / BN));
+  if (Binv) OK((run_gemm<A_KM, B_KN>(c, nb, np / BN, X, np, X, np, np, KR_UPPER, TS_ALL, epi_store(Binv, np, false))));
   return AGP_OK;
 }
 
@@ -1012,10 +1085,6 @@ __global__ void build_Lbar_kernel(const double* V, const double* X2, const doubl
   out[(int64_t)r * Mp + cidx] = v;
 }
 
-__global__ void set_diag_kernel(double* A, int n, int64_t ld, double v) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n) A[(int64_t)i * ld + i] = v;
-}
 __global__ void axpby_kernel(double a, const double* x, double b, const double* y, double* out, int64_t n) {
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
     out[i] = a * x[i] + (y ? b * y[i] : 0.0);
@@ -1087,6 +1156,27 @@ static void write_component_grads(const KernelParams& kp, const double* h_theta,
   }
 }
 
+// The kernel-parameter fields of g (agp_svgp_grads or agp_laplace_result) from theta.  scal: the SVGP's reduced scalars, whose SC_DKXX,
+// SC_DC and SC_DS terms (marginal variances) are added; nullptr where there are none (not zeros: theta + 0.0 would turn a -0.0 into +0.0).
+template <class Grads>
+static void write_kernel_grads(const KernelParams& kp, const double* h_theta, const double* scal, const Grads* g) {
+  const int D = kp.D;
+  if (g->dvariance) *g->dvariance = scal ? h_theta[0] + scal[SC_DKXX] : h_theta[0];
+  if (g->dlinear_c) *g->dlinear_c = scal ? h_theta[1] + scal[SC_DC] : h_theta[1];
+  if (g->dinv_lengthscale) {
+    const bool linear = kp.kind == AGP_KERNEL_LINEAR;
+    auto ds = [&](int d) { return scal ? h_theta[2 + d] + (linear ? scal[SC_DS + d] : 0.0) : h_theta[2 + d]; };
+    if (!kp.ard) {
+      double s = 0.0;
+      for (int d = 0; d < D; d++) s += ds(d);
+      g->dinv_lengthscale[0] = s;
+    } else {
+      for (int d = 0; d < D; d++) g->dinv_lengthscale[d] = ds(d);
+    }
+  }
+  if (kernel_is_composite(kp.kind)) write_component_grads(kp, h_theta, D, scal ? scal[SC_DKXX] : 0.0, g->dcomp_variance, g->dcomp_inv_lengthscale);
+}
+
 static int32_t resolve_params(const agp_svgp_params* p, SvgpState& st) {
   if (!p) return fail(AGP_ERR_INVALID, "params is NULL");
   if (p->M < 1 || p->D < 1 || !p->Z || !p->m || !p->Lq) return fail(AGP_ERR_INVALID, "params: M, D, Z, m, Lq are required");
@@ -1097,7 +1187,6 @@ static int32_t resolve_params(const agp_svgp_params* p, SvgpState& st) {
   st.D = p->D;
   st.Mp = (int)round_up(p->M, BM);
   st.nb = st.Mp / BM;
-  st.n_scale = p->kernel.n_scale;
   st.centered = p->parametrization == AGP_CENTERED;
   st.mean_const = p->mean_const;
   st.jitter = p->jitter;
@@ -1145,7 +1234,7 @@ static int32_t resolve_params(const agp_svgp_params* p, SvgpState& st) {
 
 // Float32 mode: hi / lo planes of the once-per-step operands of the tcgen05 stages -- Bt (column-major memory = the [j][l] operand of
 // S2, row-major memory = the [i][j] operand of S4) and the explicit inverse Linv = Lk^-1 (a block TRSM on the identity, as the Laplace
-// pullback builds B^-1), transposed to the [j][i] operand of S5.
+// pullback builds B^-1: factor_inverse), transposed to the [j][i] operand of S5.
 static int32_t prepare_f32_operands(agp_ctx* c) {
   const int Mp = c->st.Mp;
   const int64_t MM = (int64_t)Mp * Mp;
@@ -1163,12 +1252,8 @@ static int32_t prepare_f32_operands(agp_ctx* c) {
   };
   OK(split(c->Bt_cm.p, c->fBtc));
   OK(split(c->Bt_rm.p, c->fBtr));
-  // W1 (row-major) = I, W1 <- Lk^-1 W1, W2 = W1^T
-  OK(fill(c, c->W1.p, MM, 0.0));
-  set_diag_kernel<<<(Mp + 255) / 256, 256, 0, c->stream>>>(c->W1.p, Mp, Mp, 1.0);
-  LAUNCHED(c);
-  KCHECK();
-  OK(solve_lk<TR_RHS_FWD>(c, c->W1.p, Mp, Mp / BN));
+  // W1 (row-major) = Lk^-1, W2 = W1^T
+  OK(factor_inverse(c, c->Lt.p, c->st.nb, c->W1.p));
   // Linv itself (rows l, k = l' contiguous) as seven slice planes: the B operand of the INT8 forward solve (f32sweep.cuh EpiE1)
   OK(c->qLi7.ensure((i8e::S * MM + 7) / 8));
   OK(c->sLi7.ensure(Mp));
@@ -1192,12 +1277,8 @@ static int32_t prepare_step(agp_ctx* c, const agp_svgp_params* p) {
   st.sweep_pending = false;
   OK(resolve_params(p, st));
   CU(cudaSetDevice(c->device));
-  const int M = st.M, Mp = st.Mp, D = st.D, nb = st.nb;
+  const int M = st.M, Mp = st.Mp, nb = st.nb;
   const int64_t MM = (int64_t)Mp * Mp;
-  OK(c->z.ensure((int64_t)Mp * D));
-  OK(c->zs.ensure((int64_t)Mp * D));
-  OK(c->zn.ensure(Mp));
-  OK(c->zsp.ensure((int64_t)Mp * (kuf_dp(D) + 2)));
   OK(c->mvec.ensure(Mp));
   OK(c->mt.ensure(Mp));
   OK(c->vec64.ensure((int64_t)Mp * 64));
@@ -1212,8 +1293,6 @@ static int32_t prepare_step(agp_ctx* c, const agp_svgp_params* p) {
   for (int j = 0; j < M; j++)
     if (!(p->Lq[(int64_t)j * ldq + j] > 0.0))
       return fail(AGP_ERR_DOMAIN, "q.Sigma Cholesky factor has a non-positive diagonal entry at %d (logdet would throw)", j + 1);
-  CU(cudaMemsetAsync(c->z.p, 0, sizeof(double) * Mp * D, c->stream));
-  CU(cudaMemcpyAsync(c->z.p, p->Z, sizeof(double) * M * D, cudaMemcpyHostToDevice, c->stream));
   CU(cudaMemcpyAsync(c->mvec.p, st.h_m.data(), sizeof(double) * Mp, cudaMemcpyHostToDevice, c->stream));
   // (Lq is uploaded further down, on its own stream, behind the factorisation of Kuu)
   if (st.lp.method == AGP_EXPECT_GAUSS_HERMITE && st.lp.ngh > 0) {
@@ -1223,12 +1302,8 @@ static int32_t prepare_step(agp_ctx* c, const agp_svgp_params* p) {
     st.lp.gh = c->ghbuf.p;
   }
   CU(cudaMemsetAsync(c->d_flags, 0, 4 * sizeof(int), c->stream));
-  prep_z_kernel<<<(Mp + 127) / 128, 128, 0, c->stream>>>(c->z.p, c->zs.p, c->zn.p, c->zsp.p, Mp, st.kp);
-  LAUNCHED(c);
-  KCHECK();
-  build_kuu_kernel<<<dim3((Mp + 127) / 128, Mp), 128, 0, c->stream>>>(c->Kw.p, Mp, c->zs.p, c->zn.p, st.jitter, st.kp);
-  LAUNCHED(c);
-  KCHECK();
+  OK(upload_points(c, c->z, p->Z, M, st.kp, true));
+  OK(prior_cov(c, st.kp, c->z, nullptr, st.jitter, c->Kw.p));
   OK(fill(c, c->Lk.p, MM, 0.0));
   OK(fill(c, c->Lt.p, MM, 0.0));
   OK(fill(c, c->Ut.p, MM, 0.0));
@@ -1378,9 +1453,10 @@ static int32_t ensure_sweep_workspace(agp_ctx* c, int64_t cols, bool grad) {
   return AGP_OK;
 }
 
-static int32_t run_kgrad(agp_ctx* c, const double* Kb, int64_t ld, const double* pts, int npts, int nslab, const double* Kf = nullptr,
-                         const double* DK = nullptr) {
-  const SvgpState& st = c->st;
+// Contraction of the cotangent Kb (ld) of k(z, pts) with the kernel derivatives into c->kpart (z: the inducing points or training inputs)
+static int32_t run_kgrad(agp_ctx* c, const KernelParams& kp, const PointSet& z, const double* Kb, int64_t ld, const double* pts, int npts,
+                         int nslab, const double* Kf = nullptr, const double* DK = nullptr) {
+  const int D = kp.D;
   KgradArgs a{};
   a.Kb = Kb;
   a.Kf = Kf;
@@ -1388,16 +1464,16 @@ static int32_t run_kgrad(agp_ctx* c, const double* Kb, int64_t ld, const double*
   a.ld = ld;
   a.pts = pts;
   a.npts = npts;
-  a.zs = c->zs.p;
-  a.zn = c->zn.p;
+  a.zs = z.xs.p;
+  a.zn = z.xn.p;
   a.slab = 2048;
   a.part = c->kpart.p;
-  a.stride = kgrad_stride(st.D);
-  a.Mp = st.Mp;
-  a.kp = st.kp;
-  const dim3 grid((st.M + 7) / 8, nslab);
+  a.stride = kgrad_stride(D);
+  a.Mp = z.np;
+  a.kp = kp;
+  const dim3 grid((z.n + 7) / 8, nslab);
   if (Kf) {  // stationary kinds inside the sweep: stream the stored kernel values (kgrad_stream_kernel)
-    const bool se = st.kp.kind == AGP_KERNEL_SE;
+    const bool se = kp.kind == AGP_KERNEL_SE;
 #define AGP_KSTREAM(DM)                                                                              \
   {                                                                                                  \
     const int sm = KfTile<DM>::value * (DM + 2) * 8;                                                 \
@@ -1409,34 +1485,34 @@ static int32_t run_kgrad(agp_ctx* c, const double* Kb, int64_t ld, const double*
       kgrad_stream_kernel<DM, false><<<grid, 256, sm, c->stream>>>(a);                               \
     }                                                                                                \
   }
-    if (st.D <= 4) AGP_KSTREAM(4)
-    else if (st.D <= 8) AGP_KSTREAM(8)
-    else if (st.D <= 16) AGP_KSTREAM(16)
+    if (D <= 4) AGP_KSTREAM(4)
+    else if (D <= 8) AGP_KSTREAM(8)
+    else if (D <= 16) AGP_KSTREAM(16)
     else AGP_KSTREAM(32)
 #undef AGP_KSTREAM
     LAUNCHED(c);
     KCHECK();
     return AGP_OK;
   }
-  const int smem = 256 * (kuf_dp(st.D) + 2) * 8;
+  const int smem = 256 * (kuf_dp(D) + 2) * 8;
 #define AGP_KGRAD_ONE(DM, KD)                                                                                        \
   {                                                                                                                \
     if (smem > 48 * 1024) OK((ensure_smem<kgrad_kernel<DM, 1, KD>>(c, smem)));                                      \
     kgrad_kernel<DM, 1, KD><<<grid, 256, smem, c->stream>>>(a);                                                   \
   }
 #define AGP_KGRAD_LAUNCH(DM)                                          \
-  switch (st.kp.kind) {                                               \
+  switch (kp.kind) {                                                  \
     case AGP_KERNEL_SE: AGP_KGRAD_ONE(DM, AGP_KERNEL_SE) break;       \
     case AGP_KERNEL_MATERN32: AGP_KGRAD_ONE(DM, AGP_KERNEL_MATERN32) break; \
     case AGP_KERNEL_MATERN52: AGP_KGRAD_ONE(DM, AGP_KERNEL_MATERN52) break; \
     case AGP_KERNEL_LINEAR: AGP_KGRAD_ONE(DM, AGP_KERNEL_LINEAR) break; \
     default: AGP_KGRAD_ONE(DM, AGP_KERNEL_COMPOSITE) break;           \
   }
-  if (st.D <= 4) {
+  if (D <= 4) {
     AGP_KGRAD_LAUNCH(4)
-  } else if (st.D <= 8) {
+  } else if (D <= 8) {
     AGP_KGRAD_LAUNCH(8)
-  } else if (st.D <= 16) {
+  } else if (D <= 16) {
     AGP_KGRAD_LAUNCH(16)
   } else {
     AGP_KGRAD_LAUNCH(32)
@@ -1448,18 +1524,18 @@ static int32_t run_kgrad(agp_ctx* c, const double* Kb, int64_t ld, const double*
   return AGP_OK;
 }
 
-static int32_t finish_kgrad(agp_ctx* c, int nslab, double zfac, double* dZ, double* theta) {
-  const SvgpState& st = c->st;
+// dZ and theta (kgrad_finish_kernel) from the partial sums of run_kgrad
+static int32_t finish_kgrad(agp_ctx* c, const KernelParams& kp, const PointSet& z, int nslab, double zfac, double* dZ, double* theta) {
   KgradFinishArgs a{};
   a.part = c->kpart.p;
   a.nslab = nslab;
-  a.Mp = st.Mp;
-  a.stride = kgrad_stride(st.D);
-  a.zs = c->zs.p;
+  a.Mp = z.np;
+  a.stride = kgrad_stride(kp.D);
+  a.zs = z.xs.p;
   a.zfac = zfac;
   a.dZ = dZ;
   a.theta = theta;
-  a.kp = st.kp;
+  a.kp = kp;
   kgrad_finish_kernel<<<1, 256, 0, c->stream>>>(a);
   LAUNCHED(c);
   KCHECK();
@@ -1509,7 +1585,7 @@ static TrsmArgs s1_args(agp_ctx* c, double* X, int64_t ldx, const double* pts, i
   t1.ldx = ldx;
   t1.pts = pts;
   t1.npts = npts;
-  t1.zsp = c->zsp.p;
+  t1.zsp = c->z.xsp.p;
   t1.mt = c->mt.p;
   t1.saa = c->saa.p;
   t1.sam = c->sam.p;
@@ -1771,7 +1847,7 @@ static int32_t sweep_s6(agp_ctx* c, const SweepPlan& pl, int ncols) {
 static int32_t sweep_s7(agp_ctx* c, const SweepPlan& pl, const double* pts, int npts) {
   const bool dk = pl.s7_streamed && c->st.kp.kind != AGP_KERNEL_SE;
   ProfScope ps(c, PC_KGRAD);
-  return run_kgrad(c, c->Ab.p, c->chunk_cols, pts, npts, (npts + 2047) / 2048, pl.s7_streamed ? c->Kf.p : nullptr, dk ? c->DKb.p : nullptr);
+  return run_kgrad(c, c->st.kp, c->z, c->Ab.p, c->chunk_cols, pts, npts, (npts + 2047) / 2048, pl.s7_streamed ? c->Kf.p : nullptr, dk ? c->DKb.p : nullptr);
 }
 
 // local reductions of the reverse pass's partial sums into the packed reduce buffer
@@ -1784,7 +1860,7 @@ static int32_t sweep_reduce(agp_ctx* c, const RedLayout& rl) {
   sum_slices_kernel<<<1024, 256, 0, c->stream>>>(c->Gpart.p, c->nsplit, MM, MM, c->red.p + rl.G);
   LAUNCHED(c);
   KCHECK();
-  return finish_kgrad(c, c->nslab, 1.0, c->red.p + rl.dZ, c->red.p + rl.theta);
+  return finish_kgrad(c, c->st.kp, c->z, c->nslab, 1.0, c->red.p + rl.dZ, c->red.p + rl.theta);
 }
 
 // forward (+ backward) sweep over points [offset, offset+count) of ds.  predict != 0: only S1-S3 writing mu/var.
@@ -1965,8 +2041,8 @@ extern "C" int32_t agp_svgp_finish(agp_ctx* c, double* elbo_out, agp_svgp_grads*
   // Kuu part of dZ / dtheta: contraction with k(Z, Z); both arguments move -> zfac = 2
   const int nslab_z = (M + 2047) / 2048;
   OK(fill(c, c->kpart.p, (int64_t)nslab_z * Mp * kgrad_stride(D), 0.0));
-  OK(run_kgrad(c, W4, Mp, c->z.p, M, nslab_z));
-  OK(finish_kgrad(c, nslab_z, 2.0, dZ, theta));
+  OK(run_kgrad(c, st.kp, c->z, W4, Mp, c->z.x.p, M, nslab_z));
+  OK(finish_kgrad(c, st.kp, c->z, nslab_z, 2.0, dZ, theta));
   // outputs
   std::vector<double> h_theta(theta_size(D)), h_dZ((int64_t)Mp * D), h_vec(2 * (int64_t)Mp), h_g(Mp);
   std::vector<double> h_dLq;
@@ -1998,19 +2074,7 @@ extern "C" int32_t agp_svgp_finish(agp_ctx* c, double* elbo_out, agp_svgp_grads*
     for (int i = 0; i < M; i++) go->dm[i] = st.centered ? h_vec[Mp + i] : h_g[i] - st.h_m[i];
   }
   if (go->dZ) memcpy(go->dZ, h_dZ.data(), sizeof(double) * M * D);
-  if (go->dvariance) *go->dvariance = h_theta[0] + h_scal[SC_DKXX];
-  if (go->dlinear_c) *go->dlinear_c = h_theta[1] + h_scal[SC_DC];
-  if (go->dinv_lengthscale) {
-    const bool linear = st.kp.kind == AGP_KERNEL_LINEAR;
-    if (st.n_scale == 1) {
-      double s = 0.0;
-      for (int d = 0; d < D; d++) s += h_theta[2 + d] + (linear ? h_scal[SC_DS + d] : 0.0);
-      go->dinv_lengthscale[0] = s;
-    } else {
-      for (int d = 0; d < D; d++) go->dinv_lengthscale[d] = h_theta[2 + d] + (linear ? h_scal[SC_DS + d] : 0.0);
-    }
-  }
-  if (kernel_is_composite(st.kp.kind)) write_component_grads(st.kp, h_theta.data(), D, h_scal[SC_DKXX], go->dcomp_variance, go->dcomp_inv_lengthscale);
+  write_kernel_grads(st.kp, h_theta.data(), h_scal.data(), go);
   if (go->dmean_const) *go->dmean_const = h_scal[SC_DMU] - (st.centered ? h_small[1] : 0.0);
   if (go->dlik_sigma2) *go->dlik_sigma2 = h_scal[SC_DS2];
   return AGP_OK;
@@ -2206,51 +2270,28 @@ extern "C" int32_t agp_svgp_mean_and_cov(agp_ctx* c, const agp_svgp_params* p, c
   OK(prepare_step(c, p));
   SvgpState& st = c->st;
   st.scale = 1.0;
-  const int D = st.D, Mp = st.Mp;
+  const int Mp = st.Mp;
   const int n1p = (int)round_up(n1, BM), n2p = (int)round_up(n2, BM);
   OK(ensure_sweep_workspace(c, std::max(n1p, n2p), true));
   const int64_t ldc = c->chunk_cols;
-  OK(c->px1.ensure((int64_t)n1p * D));
-  OK(c->pxs1.ensure((int64_t)n1p * D));
-  OK(c->pxn1.ensure(n1p));
   OK(c->pcov.ensure((int64_t)n1p * n2p));
   OK(c->mu_out.ensure(n1p));
   OK(c->var_out.ensure(n1p));
-  CU(cudaMemsetAsync(c->px1.p, 0, sizeof(double) * n1p * D, c->stream));
-  CU(cudaMemcpyAsync(c->px1.p, X1, sizeof(double) * n1 * D, cudaMemcpyHostToDevice, c->stream));
-  KernelParams kx = st.kp;
-  kx.M = (int)n1;
-  prep_z_kernel<<<(n1p + 127) / 128, 128, 0, c->stream>>>(c->px1.p, c->pxs1.p, c->pxn1.p, nullptr, n1p, kx);
-  LAUNCHED(c);
-  KCHECK();
-  OK(project_points(c, c->px1.p, (int)n1, n1p, c->A.p, c->C.p, ldc));
+  OK(upload_points(c, c->px1, X1, n1, st.kp, false));
+  OK(project_points(c, c->px1.x.p, (int)n1, n1p, c->A.p, c->C.p, ldc));
   if (mu1_out) {
     // the per-point stage of the sweep in prediction mode; project_points ran S2 on DMMA
-    OK(sweep_s3(c, SweepPlan{}, c->px1.p, nullptr, 0, (int)n1, n1p, true, c->mu_out.p, c->var_out.p, nullptr));
+    OK(sweep_s3(c, SweepPlan{}, c->px1.x.p, nullptr, 0, (int)n1, n1p, true, c->mu_out.p, c->var_out.p, nullptr));
     CU(cudaMemcpyAsync(mu1_out, c->mu_out.p, sizeof(double) * n1, cudaMemcpyDeviceToHost, c->stream));
   }
   const double *A2 = c->A.p, *C2 = c->C.p;
   if (cross) {
-    OK(c->px2.ensure((int64_t)n2p * D));
-    OK(c->pxs2.ensure((int64_t)n2p * D));
-    OK(c->pxn2.ensure(n2p));
-    CU(cudaMemsetAsync(c->px2.p, 0, sizeof(double) * n2p * D, c->stream));
-    CU(cudaMemcpyAsync(c->px2.p, X2, sizeof(double) * n2 * D, cudaMemcpyHostToDevice, c->stream));
-    KernelParams ky = st.kp;
-    ky.M = (int)n2;
-    prep_z_kernel<<<(n2p + 127) / 128, 128, 0, c->stream>>>(c->px2.p, c->pxs2.p, c->pxn2.p, nullptr, n2p, ky);
-    LAUNCHED(c);
-    KCHECK();
-    OK(project_points(c, c->px2.p, (int)n2, n2p, c->Ab.p, c->As.p, ldc));
+    OK(upload_points(c, c->px2, X2, n2, st.kp, false));
+    OK(project_points(c, c->px2.x.p, (int)n2, n2p, c->Ab.p, c->As.p, ldc));
     A2 = c->Ab.p;
     C2 = c->As.p;
-    cross_k_kernel<<<dim3((n1p + 127) / 128, n2p), 128, 0, c->stream>>>(c->pcov.p, n1p, c->pxs1.p, c->pxn1.p, (int)n1, c->pxs2.p, c->pxn2.p, (int)n2, n1p, st.kp);
-  } else {
-    // cov(f.prior, x): the one-argument kernelmatrix (exactly zero distances on the diagonal)
-    build_kuu_kernel<<<dim3((n1p + 127) / 128, n1p), 128, 0, c->stream>>>(c->pcov.p, n1p, c->pxs1.p, c->pxn1.p, 0.0, kx);
   }
-  LAUNCHED(c);
-  KCHECK();
+  OK(prior_cov(c, st.kp, c->px1, cross ? &c->px2 : nullptr, 0.0, c->pcov.p));
   // cov = K - A1^T A2 + C1^T C2   (SVA.jl:227 / :263)
   OK((run_gemm<A_KM, B_KN>(c, n1p / BM, n2p / BN, c->A.p, ldc, A2, ldc, Mp, KR_FULL, TS_ALL, epi_store(c->pcov.p, n1p, false, -1.0, 1.0))));
   OK((run_gemm<A_KM, B_KN>(c, n1p / BM, n2p / BN, c->C.p, ldc, C2, ldc, Mp, KR_FULL, TS_ALL, epi_store(c->pcov.p, n1p, false, 1.0, 1.0))));
@@ -2270,33 +2311,12 @@ extern "C" int32_t agp_kernel_matrix(agp_ctx* c, const agp_kernel* k, int32_t D,
   if (n2 < 1 || n1 > AGP_MAX_COV_POINTS || n2 > AGP_MAX_COV_POINTS) return fail(AGP_ERR_INVALID, "agp_kernel_matrix: 1 <= n <= %lld", (long long)AGP_MAX_COV_POINTS);
   CU(cudaSetDevice(c->device));
   KernelParams kp;
-  OK(fill_kernel_params(k, D, 0, kp));
-  OK(c->px1.ensure(n1 * D));
-  OK(c->pxs1.ensure(n1 * D));
-  OK(c->pxn1.ensure(n1));
-  OK(c->pcov.ensure(n1 * n2));
-  CU(cudaMemcpyAsync(c->px1.p, X1, sizeof(double) * n1 * D, cudaMemcpyHostToDevice, c->stream));
-  kp.M = (int)n1;
-  prep_z_kernel<<<(int)((n1 + 127) / 128), 128, 0, c->stream>>>(c->px1.p, c->pxs1.p, c->pxn1.p, nullptr, (int)n1, kp);
-  LAUNCHED(c);
-  KCHECK();
-  if (cross) {
-    OK(c->px2.ensure(n2 * D));
-    OK(c->pxs2.ensure(n2 * D));
-    OK(c->pxn2.ensure(n2));
-    CU(cudaMemcpyAsync(c->px2.p, X2, sizeof(double) * n2 * D, cudaMemcpyHostToDevice, c->stream));
-    KernelParams ky = kp;
-    ky.M = (int)n2;
-    prep_z_kernel<<<(int)((n2 + 127) / 128), 128, 0, c->stream>>>(c->px2.p, c->pxs2.p, c->pxn2.p, nullptr, (int)n2, ky);
-    LAUNCHED(c);
-    KCHECK();
-    cross_k_kernel<<<dim3((int)((n1 + 127) / 128), (int)n2), 128, 0, c->stream>>>(c->pcov.p, n1, c->pxs1.p, c->pxn1.p, (int)n1, c->pxs2.p, c->pxn2.p, (int)n2, (int)n1, kp);
-  } else {
-    build_kuu_kernel<<<dim3((int)((n1 + 127) / 128), (int)n1), 128, 0, c->stream>>>(c->pcov.p, (int)n1, c->pxs1.p, c->pxn1.p, 0.0, kp);
-  }
-  LAUNCHED(c);
-  KCHECK();
-  CU(cudaMemcpyAsync(K_out, c->pcov.p, sizeof(double) * n1 * n2, cudaMemcpyDeviceToHost, c->stream));
+  OK(fill_kernel_params(k, D, (int)n1, kp));
+  OK(upload_points(c, c->px1, X1, n1, kp, false));
+  if (cross) OK(upload_points(c, c->px2, X2, n2, kp, false));
+  OK(c->pcov.ensure((int64_t)c->px1.np * (cross ? c->px2.np : c->px1.np)));
+  OK(prior_cov(c, kp, c->px1, cross ? &c->px2 : nullptr, 0.0, c->pcov.p));
+  CU(cudaMemcpy2DAsync(K_out, sizeof(double) * n1, c->pcov.p, sizeof(double) * c->px1.np, sizeof(double) * n1, n2, cudaMemcpyDeviceToHost, c->stream));
   CU(cudaStreamSynchronize(c->stream));
   return AGP_OK;
 }

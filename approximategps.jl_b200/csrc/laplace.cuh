@@ -390,11 +390,4 @@ __global__ void lap_kbar_kernel(const double* Binv, int64_t ld, int n, int np, c
   Kbar[(int64_t)j * ld + i] = out;
 }
 
-// identity (row-major [np][np]) as the right-hand side of the explicit inverse
-__global__ void lap_eye_kernel(double* X, int np) {
-  const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-  if (i >= (int64_t)np * np) return;
-  X[i] = (i / np == i % np) ? 1.0 : 0.0;
-}
-
 }  // namespace agp

@@ -91,28 +91,45 @@ def test_kernelmatrix_and_prediction(agp):
         assert rel_err(mu, rmu) < 1e-10 and rel_err(var, rvar) < 1e-10
 
 
-@pytest.mark.parametrize("op", ["sum", "product"])
+@pytest.mark.parametrize("op", ["sum", "product", "se_ard", "linear"])
 def test_laplace_sum_product(agp, op):
+    # (se_ard / linear, at D = 3: the per-dimension inverse lengthscales and LinearKernel's offset in the Laplace kernel gradient)
     X, y = olap.generate_data()
-    comps = (("se", 1.5, 0.8), ("matern52", 0.6, 2.5))
-    k = ok.Kernel(op, 2.0, np.array([1.2]), 0.0, comps)
+    rng = np.random.default_rng(17)
+    Xn = np.linspace(-1.0, 8.0, 37)
+    if op in ("sum", "product"):
+        comps = (("se", 1.5, 0.8), ("matern52", 0.6, 2.5))
+        k = ok.Kernel(op, 2.0, np.array([1.2]), 0.0, comps)
+        kd = _device_kernel(agp, op, comps, 2.0, np.array([1.2]))
+    else:
+        X = np.column_stack([X, rng.uniform(0.0, 4.0, size=(len(y), 2))])
+        Xn = rng.uniform(-1.0, 5.0, size=(37, 3))
+        if op == "se_ard":
+            inv = np.array([1.2, 0.7, 1.6])
+            k, kd = ok.Kernel(ok.SE, 2.0, inv), 2.0 * agp.ARDTransform(agp.SqExponentialKernel(), inv)
+        else:
+            k, kd = ok.Kernel(ok.LINEAR, 0.5, np.array([0.8]), 0.3), 0.5 * agp.ScaleTransform(agp.LinearKernel(0.3), 0.8)
     lik = ol.Likelihood(ol.BERNOULLI_LOGIT)
     K = ok.kernelmatrix(k, X) + 1e-8 * np.eye(len(y))
     lml, K_bar, f_opt, steps = olap.lml_and_grad_K(lik, y, K)
-    _, _, kg = ok.kernelmatrix_pullback(k, X, None, K_bar)
-    f = agp.GP(_device_kernel(agp, op, comps, 2.0, np.array([1.2])))
+    dX, _, kg = ok.kernelmatrix_pullback(k, X, None, K_bar)
+    f = agp.GP(kd)
     lfx = agp.LatentGP(f, agp.BernoulliLikelihood(), 1e-8)(X)
     r = agp.laplace_approx_lml_and_gradient(agp.LaplaceApproximation(), lfx, y)
     errs = dict(lml=abs(r.lml - lml) / abs(lml), variance=rel_err(r.grad.variance, kg.variance), inv_lengthscale=rel_err(r.grad.inv_lengthscale, kg.inv_lengthscale),
-                comp_variance=rel_err(r.grad.comp_variance, kg.comp_variance), comp_inv_lengthscale=rel_err(r.grad.comp_inv_lengthscale, kg.comp_inv_lengthscale))
+                X=rel_err(r.grad.X, dX))
+    if op in ("sum", "product"):
+        errs.update(comp_variance=rel_err(r.grad.comp_variance, kg.comp_variance), comp_inv_lengthscale=rel_err(r.grad.comp_inv_lengthscale, kg.comp_inv_lengthscale))
+    if op == "linear":
+        errs.update(linear_c=rel_err(r.grad.linear_c, kg.c))
     print(f"\n[laplace kernel {op}] lml={r.lml:.12f} " + " ".join(f"{k_}={v:.1e}" for k_, v in errs.items()))
     record_parity(f"laplace kernel {op}", errs, tol=1e-8)
     assert errs["lml"] < 1e-10 and r.steps == steps
+    assert np.shape(r.grad.inv_lengthscale) == np.shape(k.inv_lengthscale)
     for k_, v in errs.items():
         assert v < 1e-8, (k_, v)
     # prediction through the cache
     post = agp.posterior(agp.LaplaceApproximation(), lfx, y)
-    Xn = np.linspace(-1.0, 8.0, 37)
     mu, var = agp.mean_and_var(post, Xn)
     cache = olap.train_intermediates(lik, y, K, f_opt)
     rmu, rvar = olap.predict_mean_and_var(k, X, cache, Xn)
